@@ -424,6 +424,8 @@ def run_gpu_arm(args):
             graph_info = {"error": str(ex)[:200]}
     clocks = sampler.stop() if sampler else None
     value = world * args.envs * args.rollout * args.steps / (ms * 1e-3)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(wl, args.dump_outputs)
 
     # ---- e2e runs on EVERY rank (it contains collectives: moment all-reduce, barriers)
     wl.env._fused_event_hook = None
@@ -481,6 +483,36 @@ def run_gpu_arm(args):
                                               + ("the reference's own classes under oracle/ref_harness.py" if kind == "reference"
                                                  else "oracle/torch_oracle.py") + " on torch CPU"}
     print(json.dumps(line), flush=True)
+
+
+DUMP_ROWS = 4096        # envs (and resets) sampled for --dump-outputs
+
+
+def dump_outputs(wl, out_dir):
+    """What the caller of the timed rollout receives after its last step, as DIR/<name>.npy: the last env-step's
+    observations, privileged observations, rewards, reset / time-out flags, the reset count, reset ids with their
+    terminal privileged rows, and the rollout's returns and advantages.  Per-env outputs are taken at DUMP_ROWS envs and
+    the reset outputs at DUMP_ROWS resets, picked by a fixed seed and stored too (`env_rows`, `reset_rows`), so two builds
+    are compared on the same rows whatever --envs is: about 13 MB at --rollout 24.  Integer and boolean outputs are
+    stored as float64 (exact)."""
+    import numpy as np
+    env, st = wl.env, wl.storage
+    torch.cuda.synchronize()
+
+    def sample(count):
+        return torch.randperm(count, generator=torch.Generator().manual_seed(0))[:DUMP_ROWS].sort().values
+
+    rows = sample(env.num_envs)
+    n_reset = int(env._n_reset.item())
+    reset_rows = sample(n_reset)
+    out = {"env_rows": rows, "obs_buf": env.obs_buf.cpu()[rows], "privileged_obs_buf": env.privileged_obs_buf.cpu()[rows],
+           "rew_buf": env.rew_buf.cpu()[rows], "reset_buf": env.reset_buf.cpu()[rows], "time_out_buf": env.time_out_buf.cpu()[rows],
+           "n_reset": torch.tensor([n_reset]), "reset_rows": reset_rows, "reset_ids": env._reset_ids[:n_reset].cpu()[reset_rows],
+           "termination_privileged_obs": env._term_priv[:n_reset].cpu()[reset_rows],
+           "returns": st.returns.cpu()[:, rows], "advantages": st.advantages.cpu()[:, rows]}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in out.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), (t if t.dtype in (torch.float32, torch.float64) else t.double()).numpy())
 
 
 def measure_e2e(wl, args, world):
@@ -742,6 +774,8 @@ def main():
     ap.add_argument("--no-latency", action="store_true")
     ap.add_argument("--no-comm", action="store_true", help="N>1: leave out the gradient / statistics exchanges (attribution runs)")
     ap.add_argument("--amp", action="store_true", help="N>1: add the AMP discriminator-gradient and normaliser exchanges")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed (rank 0's shard) as DIR/<name>.npy")
     args = ap.parse_args()
     if args.impl == "reference":
         run_reference_arm(args)

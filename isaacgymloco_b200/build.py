@@ -39,7 +39,8 @@ def build(force: bool = False, verbose: bool = False) -> str:
         raise RuntimeError("nvcc failed building libhimloco_b200.so")
     if verbose:
         sys.stderr.write(proc.stderr)
-    with open(os.path.join(HERE, "csrc", "ptxas_info.txt"), "w") as f:
+    # the report of this build goes beside the library; csrc/ptxas_info.txt is the committed record and stays as it is
+    with open(os.path.splitext(LIB)[0] + ".ptxas.txt", "w") as f:
         f.write(proc.stderr)
     return LIB
 

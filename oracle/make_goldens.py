@@ -433,6 +433,48 @@ def mint_reset():
         print(f"[golden] reset_{case['name']}: n={n} resets={len(ids)} levels moved={(out['terrain_levels'] != state['terrain_levels'].numpy()).sum()}")
 
 
+def cfg_record(hc):
+    """What tests/test_cpu_host.py compares of a HotPathCfg, JSON-safe and exact (fp32 fields as their double values):
+    every HlCfg field, the reward table, the episode-sum rows, the noise vector and the reset / resampling ranges."""
+    import ctypes
+    import dataclasses
+    import json
+    c = hc.to_c()
+    fields = {}
+    for name, _ in C.HlCfg._fields_:
+        v = getattr(c, name)
+        fields[name] = list(v) if isinstance(v, ctypes.Array) else v
+    names, scales = hc.active_terms()
+    rec = dict(hlcfg=fields, terms=list(names), scales=[float(x) for x in scales], episode_sum_names=list(hc.episode_sum_names()),
+               noise_scale_vec=[float(x) for x in hc.noise_scale_vec()], reset=dataclasses.asdict(hc.reset))
+    return json.loads(json.dumps(rec))
+
+
+def dof_record(reference_root):
+    """aliengo.urdf's revolute-joint limits (LR:565-580 read them through Isaac Gym's asset loader) and the reference's
+    default joint angles, keyed by joint name."""
+    import xml.etree.ElementTree as ET
+    root = ET.parse(os.path.join(reference_root, "legged_gym", "resources", "robots", "aliengo", "urdf", "aliengo.urdf")).getroot()
+    limits = {j.get("name"): {k: float(v) for k, v in j.find("limit").attrib.items()}
+              for j in root.findall("joint") if j.get("type") == "revolute"}
+    dflt = {k: float(v) for k, v in H.reference_cfg("flat").init_state.default_joint_angles.items()}
+    return dict(limits=limits, default_joint_angles=dflt)
+
+
+REFERENCE_CFG_TASKS = ("flat", "stairs", "amp", "recover")
+
+
+def mint_reference_cfg():
+    """tests/golden/reference_cfg.json: cfg_record() of from_reference_cfg() for each of the reference's AlienGo*Cfg
+    classes, and dof_record() of its URDF."""
+    import json
+    out = {task: cfg_record(C.from_reference_cfg(H.reference_cfg(task), num_envs=4096, sim_dt=0.005)) for task in REFERENCE_CFG_TASKS}
+    out["aliengo_dof"] = dof_record(H.REFERENCE_ROOT)
+    with open(os.path.join(GOLDEN_DIR, "reference_cfg.json"), "w") as f:
+        json.dump(out, f, indent=1, sort_keys=True)
+        f.write("\n")
+
+
 def main():
     assert H.reference_available(), "run in the build container (needs /root/reference)"
     os.makedirs(GOLDEN_DIR, exist_ok=True)
@@ -445,6 +487,7 @@ def main():
     mint_replay()
     mint_amp()
     mint_reset()
+    mint_reference_cfg()
 
 
 if __name__ == "__main__":

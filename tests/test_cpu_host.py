@@ -130,54 +130,59 @@ def test_mocap_binary_cache_round_trip(tmp_path):
             np.testing.assert_array_equal(fr[:, :49].astype(np.float32), gold[f"clip{i}"])
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/legged_gym"), reason="needs the reference's config classes (build container only)")
+def _reference_cfg_golden():
+    """tests/golden/reference_cfg.json: what the reference's config classes and URDF give (oracle/make_goldens.py::
+    mint_reference_cfg), stored so the comparisons below run without the reference sources."""
+    import json
+    with open(os.path.join(ROOT, "tests", "golden", "reference_cfg.json")) as f:
+        return json.load(f)
+
+
 @pytest.mark.parametrize("task", ["flat", "stairs", "amp", "recover"])
 def test_presets_equal_the_reference_config_classes(task):
     """config.aliengo(task) (the constants that travel to the GPU box) == from_reference_cfg() of the
-    reference's own AlienGo*Cfg class: every field of the C struct, the reward table and the noise vector."""
-    import ctypes
+    reference's own AlienGo*Cfg class: every field of the C struct, the reward table, the noise vector and the
+    reset_idx / resampling / domain-rand ranges.  Against the stored record, and against the reference's classes
+    themselves where its sources are present."""
     from oracle import ref_harness as H
+    from oracle.make_goldens import cfg_record
     from isaacgymloco_b200 import config as C
-    rc = H.reference_cfg(task)
-    a = C.from_reference_cfg(rc, num_envs=4096, sim_dt=0.005)
-    b = C.aliengo(task, num_envs=4096)
-    ca, cb = a.to_c(), b.to_c()
-    for name, _ in C.HlCfg._fields_:
-        va, vb = getattr(ca, name), getattr(cb, name)
-        if isinstance(va, ctypes.Array):
-            va, vb = list(va), list(vb)
-        assert va == vb, name
-    (na, sa), (nb, sb) = a.active_terms(), b.active_terms()
-    assert list(na) == list(nb) and np.array_equal(np.asarray(sa), np.asarray(sb))
-    assert list(a.episode_sum_names()) == list(b.episode_sum_names())
-    assert np.array_equal(np.asarray(a.noise_scale_vec()), np.asarray(b.noise_scale_vec()))
-    import dataclasses
-    assert dataclasses.asdict(a.reset) == dataclasses.asdict(b.reset)        # reset_idx / resampling / domain-rand ranges
+    wants = [_reference_cfg_golden()[task]]
+    if H.reference_available():
+        wants.append(cfg_record(C.from_reference_cfg(H.reference_cfg(task), num_envs=4096, sim_dt=0.005)))
+    got = cfg_record(C.aliengo(task, num_envs=4096))
+    for want in wants:
+        for name, _ in C.HlCfg._fields_:
+            assert got["hlcfg"][name] == want["hlcfg"][name], name
+        for k in ("terms", "scales", "episode_sum_names", "noise_scale_vec", "reset"):
+            assert got[k] == want[k], k
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/legged_gym"), reason="needs the reference's URDF (build container only)")
 def test_aliengo_dof_constants_equal_the_urdf():
     """The joint limits / efforts / velocities the reference reads through Isaac Gym's asset loader
     (LR:565-580) come from aliengo.urdf; the constants in config.py must be those numbers, in the
-    reference's DOF order (FL, FR, RL, RR x hip, thigh, calf: LR:1145)."""
-    import xml.etree.ElementTree as ET
+    reference's DOF order (FL, FR, RL, RR x hip, thigh, calf: LR:1145).  Against the stored record, and
+    against the URDF itself where the reference sources are present."""
     from oracle import ref_harness as H
+    from oracle.make_goldens import dof_record
     from isaacgymloco_b200 import config as C
-    root = ET.parse("/root/reference/legged_gym/resources/robots/aliengo/urdf/aliengo.urdf").getroot()
-    lim = {j.get("name"): j.find("limit").attrib for j in root.findall("joint") if j.get("type") == "revolute"}
-    rc = H.reference_cfg("flat")
+    sources = [_reference_cfg_golden()["aliengo_dof"]]
+    if H.reference_available():
+        sources.append(dof_record(H.REFERENCE_ROOT))
     cfg = C.aliengo("flat")
     cfg.soft_dof_pos_limit = 1.0        # raw limits
     t = cfg.dof_tables()
-    k = 0
-    for leg in ("FL", "FR", "RL", "RR"):
-        for joint in ("hip", "thigh", "calf"):
-            a = lim[f"{leg}_{joint}_joint"]
-            assert np.float32(a["effort"]) == t["torque_limits"][k]
-            assert np.float32(a["velocity"]) == t["dof_vel_limits"][k]
-            np.testing.assert_allclose([t["dof_pos_lo"][k], t["dof_pos_hi"][k]], [float(a["lower"]), float(a["upper"])], rtol=1e-6)
-            assert np.float32(rc.init_state.default_joint_angles[f"{leg}_{joint}_joint"]) == t["default_dof_pos"][k]
-            k += 1
+    for src in sources:
+        lim, dflt = src["limits"], src["default_joint_angles"]
+        k = 0
+        for leg in ("FL", "FR", "RL", "RR"):
+            for joint in ("hip", "thigh", "calf"):
+                a = lim[f"{leg}_{joint}_joint"]
+                assert np.float32(a["effort"]) == t["torque_limits"][k]
+                assert np.float32(a["velocity"]) == t["dof_vel_limits"][k]
+                np.testing.assert_allclose([t["dof_pos_lo"][k], t["dof_pos_hi"][k]], [a["lower"], a["upper"]], rtol=1e-6)
+                assert np.float32(dflt[f"{leg}_{joint}_joint"]) == t["default_dof_pos"][k]
+                k += 1
 
 
 @pytest.mark.skipif(not os.path.isdir("/root/reference/legged_gym"), reason="needs the reference sources (build container only)")
