@@ -291,7 +291,9 @@ typedef struct HlReset {
   int32_t n_terrain_types;         /* columns of terrain_origins */
   int32_t parts;                   /* 0 = everything; else HL_RESET_* bits: only those parts (the individual reset hooks) */
   int32_t pad_;
-  int64_t num_envs_global;         /* for the high-speed slice env_id < 0.2 * num_envs (LR:649) */
+  int64_t num_envs_global;         /* all shards together */
+  int64_t high_vel_envs;           /* size of the high-speed command slice: global env ids < high_vel_envs take it (LR:649,
+                                      `env_ids < num_envs * 0.2`, counted on the host with the reference's own expression) */
   float base_init_state[13];       /* LR:1160-1161 */
   float pos_range[6];              /* x lo,hi, y lo,hi, z lo,hi */
   float rot_range[6];              /* roll, pitch, yaw lo,hi */
@@ -299,7 +301,6 @@ typedef struct HlReset {
   float dof_pos_ratio[2], dof_vel_range[2];
   float kp_range[2], kd_range[2], motor_strength_range[2];
   float cmd_lin_vel_x[2], cmd_lin_vel_y[2], cmd_ang_vel_yaw[2], cmd_heading[2];   /* self.command_ranges (they move with the curriculum) */
-  float high_vel_frac;             /* 0.2 */
   float env_length, max_episode_length_s;   /* LR:858,860 */
   /* device buffers the re-draws write (the env's own tensors) */
   float* root_states;              /* (N,13) */

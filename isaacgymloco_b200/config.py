@@ -139,15 +139,24 @@ class HlReset(ctypes.Structure):
         "struct_bytes", "custom_origins", "has_pos_range", "has_rot_range", "vel_range_is_dict", "randomize_dof_pos",
         "randomize_dof_vel", "randomize_kp", "randomize_kd", "randomize_motor_strength", "heading_command",
         "terrain_curriculum", "max_terrain_level", "n_terrain_types", "parts", "pad_")] + [
-        ("num_envs_global", ctypes.c_int64),
+        ("num_envs_global", ctypes.c_int64), ("high_vel_envs", ctypes.c_int64),
         ("base_init_state", ctypes.c_float * 13), ("pos_range", ctypes.c_float * 6), ("rot_range", ctypes.c_float * 6),
         ("vel_range", ctypes.c_float * 12), ("dof_pos_ratio", ctypes.c_float * 2), ("dof_vel_range", ctypes.c_float * 2),
         ("kp_range", ctypes.c_float * 2), ("kd_range", ctypes.c_float * 2), ("motor_strength_range", ctypes.c_float * 2),
         ("cmd_lin_vel_x", ctypes.c_float * 2), ("cmd_lin_vel_y", ctypes.c_float * 2), ("cmd_ang_vel_yaw", ctypes.c_float * 2),
-        ("cmd_heading", ctypes.c_float * 2), ("high_vel_frac", ctypes.c_float), ("env_length", ctypes.c_float),
+        ("cmd_heading", ctypes.c_float * 2), ("env_length", ctypes.c_float),
         ("max_episode_length_s", ctypes.c_float)] + [(n, ctypes.c_void_p) for n in (
         "root_states", "dof_state", "commands", "env_origins", "terrain_origins", "terrain_levels", "terrain_types",
         "kp_factors", "kd_factors", "motor_strength_factors", "uniforms", "means_out", "means_ws")]
+
+
+def high_vel_env_count(num_envs: int) -> int:
+    """Size of the high-speed command slice of _resample_commands: the global env ids with `env_ids < num_envs * 0.2`
+    (LR:649), computed once per env object.  torch compares the int64 ids with the Python float in fp32, so the count
+    is the number of ids below the fp32-rounded product (ids are exact in fp32 below 2**24).  The kernels compare the
+    id with this integer; a product with the fp32 0.2f takes one env too many whenever num_envs is a multiple of 5."""
+    n = int(num_envs)
+    return min(n, math.ceil(float(np.float32(n * 0.2))))
 
 
 def _f32(x) -> float:

@@ -408,7 +408,7 @@ __device__ __forceinline__ void hl_resample_env(const HlReset& r, const ResetUni
   float c1 = ru.range(37, r.cmd_lin_vel_y);                        // LR:642
   const float c3 = ru.range(38, r.heading_command ? r.cmd_heading : r.cmd_ang_vel_yaw);   // LR:643-646
   const float hv = ru.range(39, r.cmd_lin_vel_x);
-  if ((double)gid < (double)r.num_envs_global * (double)r.high_vel_frac) {   // LR:649-653 (env_ids < num_envs * 0.2)
+  if (gid < r.high_vel_envs) {   // LR:649-653 (env_ids < num_envs * 0.2)
     c0 = hv;
     c1 *= fabsf(c0) < 1.0f ? 1.0f : 0.0f;     // norm of a 1-vector
   }
@@ -878,7 +878,7 @@ __global__ void __launch_bounds__(256) hl_resample_kernel(HlCfg c, HlEnvBuffers 
   float c1 = (r.cmd_lin_vel_y[1] - r.cmd_lin_vel_y[0]) * u[1] + r.cmd_lin_vel_y[0];
   const float* lohi = r.heading_command ? r.cmd_heading : r.cmd_ang_vel_yaw;
   const float c3 = (lohi[1] - lohi[0]) * u[2] + lohi[0];
-  if ((double)gid < (double)r.num_envs_global * (double)r.high_vel_frac) {
+  if (gid < r.high_vel_envs) {
     c0 = (r.cmd_lin_vel_x[1] - r.cmd_lin_vel_x[0]) * u[3] + r.cmd_lin_vel_x[0];
     c1 *= fabsf(c0) < 1.0f ? 1.0f : 0.0f;
   }
@@ -1417,7 +1417,7 @@ struct FusedArgs {
   int cf_stride, need_ldp, need_ltq, want_base;
   long long rs_interval;  // > 0: resample the commands of envs whose incremented episode length hits the interval (LR:612-613)
   int rs_heading;
-  double rs_hi_envs;      // num_envs * 0.2 (LR:649)
+  long long rs_hi_envs;   // HlReset::high_vel_envs (LR:649)
   float rs_lin_vel_x[2], rs_lin_vel_y[2], rs_third[2];   // third = heading range (heading_command) or yaw-rate range
   const float* rs_uniforms;   // (N, HL_RESET_NU) or nullptr => Philox stream 2
   int hist_pf;            // bulk-prefetch the tile's obs-history slab into L2 (obs_buf_in 16-B aligned)
@@ -1441,7 +1441,7 @@ __device__ __forceinline__ void hl_fused_resample(const FusedArgs& fa, const HlE
   float c0 = (1.0f - (-1.0f)) * u[0] + (-1.0f);
   float c1 = (fa.rs_lin_vel_y[1] - fa.rs_lin_vel_y[0]) * u[1] + fa.rs_lin_vel_y[0];
   const float c3 = (fa.rs_third[1] - fa.rs_third[0]) * u[2] + fa.rs_third[0];
-  if ((double)gid < fa.rs_hi_envs) {
+  if (gid < fa.rs_hi_envs) {
     c0 = (fa.rs_lin_vel_x[1] - fa.rs_lin_vel_x[0]) * u[3] + fa.rs_lin_vel_x[0];
     c1 *= fabsf(c0) < 1.0f ? 1.0f : 0.0f;
   }
@@ -1582,7 +1582,7 @@ extern "C" int hl_post_physics_fused(const HlCfg* cfg, const HlEnvBuffers* bufs,
       HL_CHECK_ARG(r->struct_bytes == (int)sizeof(HlReset), "resample_host: HlReset size mismatch");
       fa.rs_interval = b.resample_interval;
       fa.rs_heading = r->heading_command;
-      fa.rs_hi_envs = (double)r->num_envs_global * (double)r->high_vel_frac;
+      fa.rs_hi_envs = (long long)r->high_vel_envs;
       fa.rs_lin_vel_x[0] = r->cmd_lin_vel_x[0]; fa.rs_lin_vel_x[1] = r->cmd_lin_vel_x[1];
       fa.rs_lin_vel_y[0] = r->cmd_lin_vel_y[0]; fa.rs_lin_vel_y[1] = r->cmd_lin_vel_y[1];
       const float* third = r->heading_command ? r->cmd_heading : r->cmd_ang_vel_yaw;

@@ -22,8 +22,8 @@ One env-step (post_physics_step_device, no host sync, CUDA-graph capturable):
     hl_reset_and_fixup         reset_idx (curriculum, dof / root / command re-draws, gain factors, buffer zeroing,
                                extras["episode"] means) + re-scan, obs slot 0 and roll of the reset envs
                                                                                     LR:229-241,288-361
-post_physics_step() adds the one `.item()` its return signature needs, after everything is queued, and hands the
-re-drawn rows to PhysX (`set_*_state_tensor_indexed`).
+post_physics_step() adds the one `.item()` its return signature needs, after everything is queued, hands the
+re-drawn rows to PhysX (`set_*_state_tensor_indexed`) and, on a step with resets, builds extras["episode"].
 """
 import ctypes
 import math
@@ -33,7 +33,7 @@ from typing import Callable, Dict, Optional
 import torch
 
 from . import _lib as L
-from .config import HlReset, HotPathCfg
+from .config import HlReset, HotPathCfg, high_vel_env_count
 
 
 class FusedLeggedRobot:
@@ -397,6 +397,7 @@ class FusedLeggedRobot:
                                        ang_vel_yaw=list(R.ang_vel_yaw), heading=list(R.heading))
         if not hasattr(self, "init_done"):
             self.init_done = True
+        self._high_vel_envs = high_vel_env_count(self.cfg_hot.num_envs)         # LR:649, keyed by the global env id
         self._reset_uniforms = None           # parity mode: (N, RESET_NU) pre-drawn U[0,1)
         self._episode_means = z(max(self._episode_sums_buf.shape[0], 1))
         self._means_ws = z(self._episode_sums_buf.shape[0] + 1, dtype=torch.float64)      # zeroed once; the kernel re-arms it
@@ -438,8 +439,8 @@ class FusedLeggedRobot:
         cr = self.command_ranges
         r.cmd_lin_vel_x[:], r.cmd_lin_vel_y[:] = cr["lin_vel_x"], cr["lin_vel_y"]
         r.cmd_ang_vel_yaw[:], r.cmd_heading[:] = cr["ang_vel_yaw"], cr["heading"]
-        r.high_vel_frac = 0.2
         r.num_envs_global = self.cfg_hot.num_envs
+        r.high_vel_envs = self._high_vel_envs
         has_cur = R.terrain_curriculum and self.init_done and self.terrain_origins is not None and self.terrain_types is not None
         r.terrain_curriculum = int(bool(has_cur))
         r.max_terrain_level = int(self.max_terrain_level)
@@ -569,26 +570,26 @@ class FusedLeggedRobot:
         if R.disturbance and self.common_step_counter % self.cfg_hot.disturbance_interval == 0:
             self._disturbance_robots()
 
-    def _log_episode(self, in_kernel=False):
-        """extras of reset_idx (LR:344-359); the masked means come from the reset launch itself (`in_kernel`) or from
-        one launch over the device id list."""
-        if not in_kernel:
-            L.check(L.lib.hl_episode_means(L.ptr(self._episode_sums_buf), L.ptr(self.episode_length_buf), L.ptr(self._reset_ids),
-                                           L.ptr(self._n_reset), self._episode_sums_buf.shape[0], self.num_envs, float(self.dt), 1,
-                                           L.ptr(self._episode_means), L.stream()))
-        ep = self.extras.setdefault("episode", {})
-        for k, key in enumerate(self.episode_sums.keys()):
-            ep["rew_" + key] = self._episode_means[k]
+    def _log_episode(self):
+        """extras of reset_idx (LR:344-359) after a kernel-chain step with resets.  Like the reference, every such step
+        gets a fresh dict of fresh tensors (a runner that keeps infos["episode"] of every step sees each step's own
+        means) and a step without resets leaves the previous dict in place.  The masked means come from the reset launch
+        itself; terrain_level is taken from the post-reset levels, after this step's curriculum moves (LR:352-353)."""
+        means = self._episode_means.clone()
+        ep = {"rew_" + key: means[k] for k, key in enumerate(self.episode_sums.keys())}
         if self.cfg_hot.reset.terrain_curriculum and self.terrain_origins is not None:
             ep["terrain_level"] = torch.mean(self.terrain_levels.float())
         if self.cfg_hot.reset.commands_curriculum:
             ep["max_command_x"] = self.command_ranges["lin_vel_x"][1]
+        self.extras["episode"] = ep
         self.extras["time_outs"] = self.time_out_buf
 
     def post_physics_step_device(self):
         """LR:178-247 as ONE chain of launches without a host sync (CUDA-graph capturable when no torch hook is
         overridden): returns the capacity-N id / terminal-row buffers and the device count.  post_physics_step()
-        is this plus the one `.item()` the reference's return signature needs, issued after everything is queued."""
+        is this plus the one `.item()` the reference's return signature needs, issued after everything is queued.
+        With the in-kernel reset this chain only writes the episode means to a device buffer: building
+        extras["episode"] (allocations, and only on steps with resets) is left to the caller, post_physics_step()."""
         R = self.cfg_hot.reset
         gym = getattr(self, "gym", None)
         if gym is not None:                                   # LR:187-190
@@ -634,7 +635,6 @@ class FusedLeggedRobot:
             if self._kernel_reset_ok():
                 if R.commands_curriculum and self.common_step_counter % self.max_episode_length == 0:   # LR:306-307 (1 step in 1000)
                     self.update_command_curriculum(self._reset_ids[:int(self._n_reset.item())])
-                self._log_episode(in_kernel=True)
                 r = self._reset_struct()
                 r.means_out, r.means_ws = L.ptr(self._episode_means), L.ptr(self._means_ws)
                 c, b = ctypes.byref(self._c), ctypes.byref(self._buffers())
@@ -673,6 +673,8 @@ class FusedLeggedRobot:
             ids32 = env_ids.to(torch.int32)                   # LR:713-716,817-820: hand the re-drawn rows to PhysX
             gym.set_dof_state_tensor_indexed(self.sim, self._uw(self.dof_state), self._uw(ids32), n_reset)
             gym.set_actor_root_state_tensor_indexed(self.sim, self._uw(self.root_states), self._uw(ids32), n_reset)
+        if n_reset and self._kernel_reset_ok():
+            self._log_episode()                               # LR:344-359 (the torch-hook reset_idx logs itself)
         if n_reset and getattr(self, "_reset_sets_physx", False) and hasattr(self, "refresh_actor_rigid_shape_props"):
             self.refresh_actor_rigid_shape_props(env_ids)     # LR:343: friction / restitution re-draw (PhysX actor props)
         return env_ids, term_priv[:n_reset], term_amp[:n_reset]

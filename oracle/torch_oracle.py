@@ -485,8 +485,11 @@ class OracleEnv:
         return torch.cat((self.dof_pos, self.base_lin_vel, self.base_ang_vel, self.dof_vel), dim=-1)
 
     # ------------------------------------------------------------------ the step
-    def pre_reset(self, noise):
-        """LR:193-228 minus the RNG-driven calls (_resample_commands, pushes, disturbances)."""
+    def pre_reset(self, noise, push_vel=None):
+        """LR:193-228 minus the RNG-driven calls (_resample_commands, pushes, disturbances).  `push_vel` (N,2): the
+        root xy velocities a push step's _push_robots writes (LR:627-628, 822-828), applied where
+        _post_physics_step_callback applies them (LR:607-632): after the heading command and the height scan,
+        before termination and rewards."""
         c = self.cfg
         n = self.num_envs
         self.episode_length_buf += 1
@@ -506,6 +509,8 @@ class OracleEnv:
             self.commands[:, 2] = torch.clip(0.5 * wrap_to_pi(self.commands[:, 3] - heading), -2.0, 2.0)
         if c.measure_heights:
             self.measured_heights = self._get_heights()
+        if push_vel is not None:                                    # LR:627-628
+            self.root_states[:, 7:9] = push_vel
         self.check_termination()
         self.compute_reward()
         env_ids = self.reset_buf.nonzero(as_tuple=False).flatten()

@@ -26,6 +26,23 @@ def test_library_exports_every_declared_symbol():
     assert L.lib.hl_sizeof_env_buffers() == ctypes.sizeof(L.HlEnvBuffers)
 
 
+def test_high_speed_slice_count_is_the_references():
+    """The integer the kernels compare global env ids with equals the size of the reference's slice
+    `env_ids < num_envs * 0.2` (LR:649) for every num_envs up to 300,000.  Since arange is increasing, the
+    reference's count is fixed by the comparison on the ids next to the boundary; it is checked there for every size,
+    and on the whole arange for every size up to 2,000 and for the sizes the tests and the benchmark use."""
+    from isaacgymloco_b200.config import high_vel_env_count
+    for n in range(1, 300001):
+        c = high_vel_env_count(n)
+        lo, hi = max(c - 2, 0), min(c + 2, n)
+        w = torch.arange(lo, hi) < n * 0.2            # the reference's comparison on ids lo .. hi-1
+        k = int(w.sum())
+        assert lo + k == c and (lo == 0 or bool(w[0])) and (hi == n or not bool(w[-1])), n
+    for n in list(range(1, 2001)) + [4096, 4100, 16384, 16385, 65536, 262144, 299995, 300000]:
+        assert high_vel_env_count(n) == int((torch.arange(n) < n * 0.2).sum()), n
+    assert [high_vel_env_count(n) for n in (20, 4100, 5000, 16385)] == [4, 820, 1000, 3277]
+
+
 def test_abi_guards_reject_bad_structs():
     from isaacgymloco_b200 import _lib as L
     from isaacgymloco_b200 import config as C
