@@ -156,7 +156,7 @@ typedef struct HlEnvBuffers {
   const float* noise_u45;         /* (N,45)  */
   const float* noise_u187;        /* (N,187) */
   uint64_t philox_seed;
-  uint64_t philox_offset;         /* advance by 1 per step */
+  uint64_t philox_offset;         /* advance by 1 per step (relative to *step_base when that is set) */
   int32_t* height_idx_out;        /* optional debug: (N,n_px*n_py,2) clipped (px,py) */
   float* base_height_out;         /* (N,) written by HL_ST_BASE_HEIGHT */
   /* Optional single-launch mode of hl_post_physics_fused: when reset_ids_out is non-NULL the fused
@@ -180,6 +180,10 @@ typedef struct HlEnvBuffers {
   int64_t resample_interval;
   const float* height_min3f;      /* (rows-1,cols-1) fp32 = min3 * vertical_scale from hl_terrain_prepare_f32; may be
                                    * NULL (then the fused step uses the tiled fallback kernel and height_min3) */
+  const int64_t* step_base;       /* (1,) device step counter or NULL.  Set: every Philox key uses *step_base + philox_offset
+                                   * in place of philox_offset, read by each CTA after griddepcontrol.wait -- a captured CUDA
+                                   * graph then draws fresh noise on every replay once something on the stream advances the
+                                   * counter.  NULL = the step index arrives by value in philox_offset. */
 } HlEnvBuffers;
 
 int hl_version(void);

@@ -29,7 +29,8 @@ class HlEnvBuffers(ctypes.Structure):
         ("philox_seed", c_uint64), ("philox_offset", c_uint64), ("height_idx_out", _vp),
         ("base_height_out", _vp), ("reset_ids_out", _vp), ("n_reset_out", _vp), ("term_priv_out", _vp),
         ("term_amp_out", _vp), ("term_noise_u45", _vp), ("term_noise_u187", _vp), ("fused_ws", _vp),
-        ("foot_records", _vp), ("resample_host", _vp), ("resample_interval", c_int64), ("height_min3f", _vp)]
+        ("foot_records", _vp), ("resample_host", _vp), ("resample_interval", c_int64), ("height_min3f", _vp),
+        ("step_base", _vp)]
 
 
 class HlTransition(ctypes.Structure):

@@ -199,6 +199,20 @@ __device__ __forceinline__ uint4 hl_noise_block(const HlPhiloxKeys& keys, uint64
   return hl_philox4x32_10(ctr, keys);
 }
 
+// The step index that keys every Philox stream: philox_offset, plus *step_base when the step counter lives on the
+// device (a replayed CUDA graph, which cannot take a new value by argument).  Read after griddepcontrol.wait: the op
+// that advanced the counter may be the predecessor in the stream.
+__device__ __forceinline__ unsigned long long hl_step_key(const HlEnvBuffers& b) {
+  return b.step_base ? (unsigned long long)(*b.step_base) + b.philox_offset : b.philox_offset;
+}
+// The same, read once per CTA: thread 0 loads it into `*slot` (shared memory) and the barrier publishes it; every
+// thread of the CTA must call.
+__device__ __forceinline__ uint64_t hl_step_key_cta(const HlEnvBuffers& b, unsigned long long* slot) {
+  if (threadIdx.x == 0) *slot = hl_step_key(b);
+  __syncthreads();
+  return *slot;
+}
+
 __device__ __forceinline__ unsigned hl_pick(const uint4& q, int cpt) { return cpt == 0 ? q.x : (cpt == 1 ? q.y : (cpt == 2 ? q.z : q.w)); }
 
 // Canonical mapping of one env's observation noise onto Philox blocks (stream 0 = observation,

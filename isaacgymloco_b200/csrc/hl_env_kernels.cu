@@ -203,8 +203,8 @@ __device__ __forceinline__ float warp_sum(float v) {
 // iterations 4*pass .. 4*pass+3 (point 32*it + lane takes component it&3 of block pass*32+lane).
 struct HeightNoise {
   uint4 blk;
-  __device__ __forceinline__ void refill(const HlEnvBuffers& b, unsigned long long genv, int pass, int lane, unsigned stream) {
-    blk = hl_noise_block(b.philox_seed, b.philox_offset, genv, (unsigned)(pass * 32 + lane), stream);
+  __device__ __forceinline__ void refill(const HlEnvBuffers& b, uint64_t step, unsigned long long genv, int pass, int lane, unsigned stream) {
+    blk = hl_noise_block(b.philox_seed, step, genv, (unsigned)(pass * 32 + lane), stream);
   }
   __device__ __forceinline__ float get(int it, int /*lane*/) const {
     const int cpt = it & 3;
@@ -225,8 +225,8 @@ struct ScanOut {
 };
 
 // it_mod / it_rem: this warp only handles the 32-point iterations with it % it_mod == it_rem (the
-// post-reset fix-up spreads one env over several warps); 1 / 0 = all of them.
-__device__ __forceinline__ float hl_warp_scan_env(const HlCfg& c, const HlEnvBuffers& b, const float* root,
+// post-reset fix-up spreads one env over several warps); 1 / 0 = all of them.  `step`: the Philox step key.
+__device__ __forceinline__ float hl_warp_scan_env(const HlCfg& c, const HlEnvBuffers& b, uint64_t step, const float* root,
                                                   unsigned long long genv, int lane, bool do_heights, bool want_base,
                                                   const ScanOut& o, unsigned noise_stream, int it_mod = 1, int it_rem = 0) {
   float qz, qw;
@@ -239,7 +239,7 @@ __device__ __forceinline__ float hl_warp_scan_env(const HlCfg& c, const HlEnvBuf
       HeightNoise hn;
       for (int it = 0; it * 32 < P; ++it) {
         const int p = it * 32 + lane;
-        if (o.priv_heights && !o.u187 && (it & 3) == 0) hn.refill(b, genv, it >> 2, lane, noise_stream);
+        if (o.priv_heights && !o.u187 && (it & 3) == 0) hn.refill(b, step, genv, it >> 2, lane, noise_stream);
         float u = 0.5f;
         if (o.priv_heights && c.add_noise) u = o.u187 ? (p < P ? o.u187[p] : 0.5f) : hn.get(it, lane);
         if (p < P) {
@@ -280,7 +280,7 @@ __device__ __forceinline__ float hl_warp_scan_env(const HlCfg& c, const HlEnvBuf
         if ((it % it_mod) != it_rem) continue;
         const int p = it * 32 + lane;
         const float mh = (float)hraw[it] * c.vertical_scale;
-        if (o.priv_heights && !o.u187 && (it >> 2) != pass) { pass = it >> 2; hn.refill(b, genv, pass, lane, noise_stream); }
+        if (o.priv_heights && !o.u187 && (it >> 2) != pass) { pass = it >> 2; hn.refill(b, step, genv, pass, lane, noise_stream); }
         float u = 0.5f;
         if (o.priv_heights && c.add_noise) u = o.u187 ? (p < P ? o.u187[p] : 0.5f) : hn.get(it, lane);
         if (p < P) {
@@ -383,15 +383,16 @@ __device__ __forceinline__ void hl_stage_env(float* st, const HlCfg& c, const Hl
 
 // ============================================================================= reset_idx re-draws (SURVEY.md §8f rank 2)
 // u[k] of one env: column k of its uniform vector (include/himloco_b200.h: HL_RESET_NU).  Philox mode: lane l
-// computes block l (four uniforms) of stream `stream`, keyed by (seed, offset, global env id); a shuffle hands
+// computes block l (four uniforms) of stream `stream`, keyed by (seed, step, global env id); a shuffle hands
 // column k to every lane.
 struct ResetUniforms {
   uint4 blk;
   const float* row;   // pre-drawn row or nullptr
-  __device__ __forceinline__ void init(const HlEnvBuffers& b, const HlReset& r, long long e, unsigned long long genv, int lane, unsigned stream) {
+  __device__ __forceinline__ void init(const HlEnvBuffers& b, uint64_t step, const HlReset& r, long long e, unsigned long long genv, int lane,
+                                       unsigned stream) {
     row = r.uniforms ? r.uniforms + e * HL_RESET_NU : nullptr;
     blk = make_uint4(0u, 0u, 0u, 0u);
-    if (!row && lane < (HL_RESET_NU + 3) / 4) blk = hl_noise_block(b.philox_seed, b.philox_offset, genv, (unsigned)lane, stream);
+    if (!row && lane < (HL_RESET_NU + 3) / 4) blk = hl_noise_block(b.philox_seed, step, genv, (unsigned)lane, stream);
   }
   __device__ __forceinline__ float get(int k) const {   // warp-uniform k; every lane of the warp must call
     const unsigned x = __shfl_sync(0xffffffffu, hl_pick(blk, k & 3), k >> 2);
@@ -424,10 +425,10 @@ __device__ __forceinline__ void hl_resample_env(const HlReset& r, const ResetUni
 
 // reset_idx for env e, the part that draws: terrain curriculum, dofs, root state, commands, gain factors
 // (LR:301-320,336-341).  Warp-cooperative: lanes 0-11 own one dof each, lane 0 the scalars.
-__device__ __forceinline__ void hl_reset_draw_env(const HlCfg& c, const HlEnvBuffers& b, const HlReset& r, long long e, int lane) {
+__device__ __forceinline__ void hl_reset_draw_env(const HlCfg& c, const HlEnvBuffers& b, uint64_t step, const HlReset& r, long long e, int lane) {
   const long long gid = e + c.env_id_offset;
   ResetUniforms ru;
-  ru.init(b, r, e, (unsigned long long)gid, lane, 3u);
+  ru.init(b, step, r, e, (unsigned long long)gid, lane, 3u);
   const unsigned parts = r.parts ? (unsigned)r.parts : 0xffffffffu;
   // ---- _update_terrain_curriculum (LR:845-866): pre-reset root position and commands
   if ((parts & HL_RESET_CURRICULUM) && r.terrain_curriculum && r.terrain_origins && r.terrain_types) {
@@ -524,15 +525,15 @@ __device__ __forceinline__ void hl_reset_draw_env(const HlCfg& c, const HlEnvBuf
 // One env through any subset of the stages, by one warp (or, with a split, by one warp of its group: `lead` does the
 // buffer resets, slot 0 / privileged_obs[0:51] and the roll, the others the height iterations it % it_mod == it_rem).
 // `items`: length of the id list -- the warp that completes it finalises the episode-logging means; < 0 = the caller
-// finalises them itself.  `st`: this warp's staging area (hl_warp_stage_floats floats of shared memory).
-__device__ __forceinline__ void hl_stage_one(const HlCfg& c, const HlEnvBuffers& b, const HlReset& rs, const unsigned stages, float* st,
+// finalises them itself.  `st`: this warp's staging area (hl_warp_stage_floats floats of shared memory).  `step`: the Philox step key.
+__device__ __forceinline__ void hl_stage_one(const HlCfg& c, const HlEnvBuffers& b, const uint64_t step, const HlReset& rs, const unsigned stages, float* st,
                                              const long long e, const long long n, const long long items, const int lane,
                                              const bool lead, const bool scans, const int it_mod, const int it_rem) {
   const int B = c.num_bodies;
   const int P = c.n_px * c.n_py;
   const int PD = hl_priv_dim(c);
   __syncwarp();   // the previous env's staged records are no longer read
-  if ((stages & HL_ST_RESET_DRAW) && lead) hl_reset_draw_env(c, b, rs, e, lane);   // writes the env's root / dof / command rows
+  if ((stages & HL_ST_RESET_DRAW) && lead) hl_reset_draw_env(c, b, step, rs, e, lane);   // writes the env's root / dof / command rows
   EnvView v;
   hl_stage_env(st, c, b, e, lane, (stages & HL_ST_RESET_ZERO) != 0, v);
   if ((stages & HL_ST_RESET_ZERO) && lead) {  // LR:323-329,350,361
@@ -643,7 +644,7 @@ heights_only:
     o.u187 = nullptr;
     o.clip = false;
     o.keep = myh;
-    s.base_h = hl_warp_scan_env(c, b, v.root, (unsigned long long)s.gid, lane, do_h, want_base && lead, o, 0u, it_mod, it_rem);
+    s.base_h = hl_warp_scan_env(c, b, step, v.root, (unsigned long long)s.gid, lane, do_h, want_base && lead, o, 0u, it_mod, it_rem);
     if ((stages & HL_ST_BASE_HEIGHT) && b.base_height_out && lane == 0) b.base_height_out[e] = s.base_h;
   }
   if ((stages & HL_ST_TERMINATION) && lead) {
@@ -684,7 +685,7 @@ heights_only:
       int cb, c0;
       hl_cur_noise_slot(P, cb, c0);
       if (c.add_noise && !b.noise_u45)
-        nb = hl_noise_block(b.philox_seed, b.philox_offset, (unsigned long long)s.gid, (unsigned)(cb * 32 + lane), 0u);
+        nb = hl_noise_block(b.philox_seed, step, (unsigned long long)s.gid, (unsigned)(cb * 32 + lane), 0u);
 #pragma unroll
       for (int h = 0; h < 2; ++h) {
         const int k = lane + 32 * h;
@@ -710,7 +711,7 @@ heights_only:
       for (int it = 0; it * 32 < P; ++it) {
         if ((it % it_mod) != it_rem) continue;
         const int p = it * 32 + lane;
-        if (!b.noise_u187 && (it >> 2) != pass) { pass = it >> 2; hn.refill(b, (unsigned long long)s.gid, pass, lane, 0u); }
+        if (!b.noise_u187 && (it >> 2) != pass) { pass = it >> 2; hn.refill(b, step, (unsigned long long)s.gid, pass, lane, 0u); }
         float u = 0.5f;
         if (c.add_noise) u = b.noise_u187 ? (p < P ? b.noise_u187[e * P + p] : 0.5f) : hn.get(it, lane);
         if (p < P) {
@@ -755,6 +756,8 @@ __global__ void __launch_bounds__(256, 3) hl_stage_kernel(HlCfg c, HlEnvBuffers 
   // it % (parts-1) == part-1 (scan + height part of privileged_obs): shorter dependent chains for the
   // few hundred reset envs of a step.
   hl_pdl_enter();
+  __shared__ unsigned long long s_step;
+  const uint64_t step = hl_step_key_cta(b, &s_step);
   const unsigned stages = STAGES ? STAGES : stages_rt;
   const int lane = threadIdx.x & 31;
   const long long warp0 = ((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
@@ -771,7 +774,7 @@ __global__ void __launch_bounds__(256, 3) hl_stage_kernel(HlCfg c, HlEnvBuffers 
     const int it_mod = np == 1 ? 1 : np - 1, it_rem = np == 1 ? 0 : part - 1;
     const long long e = ids ? ids[it0] : it0;
     if (e < 0 || e >= n) continue;
-    hl_stage_one(c, b, rs, stages, st, e, n, items, lane, lead, scans, it_mod, it_rem);
+    hl_stage_one(c, b, step, rs, stages, st, e, n, items, lane, lead, scans, it_mod, it_rem);
   }
 }
 
@@ -854,6 +857,8 @@ extern "C" int hl_reset_and_fixup(const HlCfg* cfg, const HlEnvBuffers* bufs, co
 __global__ void __launch_bounds__(256) hl_resample_kernel(HlCfg c, HlEnvBuffers b, HlReset r, const long long* __restrict__ ids,
                                                           const int* __restrict__ n_ids, long long interval, long long n) {
   hl_pdl_enter();
+  __shared__ unsigned long long s_step;
+  const uint64_t step = hl_step_key_cta(b, &s_step);
   const long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   long long e;
   if (ids) {
@@ -871,7 +876,7 @@ __global__ void __launch_bounds__(256) hl_resample_kernel(HlCfg c, HlEnvBuffers 
 #pragma unroll
     for (int k = 0; k < 4; ++k) u[k] = r.uniforms[e * HL_RESET_NU + 36 + k];
   } else {
-    const uint4 q = hl_noise_block(b.philox_seed, b.philox_offset, (unsigned long long)gid, 9u, ids ? 3u : 2u);
+    const uint4 q = hl_noise_block(b.philox_seed, step, (unsigned long long)gid, 9u, ids ? 3u : 2u);
     u[0] = hl_u01(q.x); u[1] = hl_u01(q.y); u[2] = hl_u01(q.z); u[3] = hl_u01(q.w);
   }
   float c0 = (1.0f - (-1.0f)) * u[0] + (-1.0f);
@@ -926,6 +931,8 @@ __global__ void __launch_bounds__(256) hl_terminal_rows_kernel(HlCfg c, HlEnvBuf
                                                                float* __restrict__ out_priv, float* __restrict__ out_amp,
                                                                long long n) {
   hl_pdl_enter();
+  __shared__ unsigned long long s_step;
+  const uint64_t step = hl_step_key_cta(b, &s_step);
   const int lane = threadIdx.x & 31;
   const long long warp0 = ((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
   const long long nwarps = ((long long)gridDim.x * blockDim.x) >> 5;
@@ -952,7 +959,7 @@ __global__ void __launch_bounds__(256) hl_terminal_rows_kernel(HlCfg c, HlEnvBuf
       int cb, c0;
       hl_cur_noise_slot(P, cb, c0);
       if (c.add_noise && !u45)
-        nb = hl_noise_block(b.philox_seed, b.philox_offset, (unsigned long long)s.gid, (unsigned)(cb * 32 + lane), 1u);
+        nb = hl_noise_block(b.philox_seed, step, (unsigned long long)s.gid, (unsigned)(cb * 32 + lane), 1u);
 #pragma unroll
       for (int h = 0; h < 2; ++h) {
         const int k = lane + 32 * h;
@@ -969,7 +976,7 @@ __global__ void __launch_bounds__(256) hl_terminal_rows_kernel(HlCfg c, HlEnvBuf
       const float rz = v.root[2];
       for (int it = 0; it * 32 < P; ++it) {
         const int p = it * 32 + lane;
-        if (!u187 && (it & 3) == 0) hn.refill(b, (unsigned long long)s.gid, it >> 2, lane, 1u);
+        if (!u187 && (it & 3) == 0) hn.refill(b, step, (unsigned long long)s.gid, it >> 2, lane, 1u);
         float u = 0.5f;
         if (c.add_noise) u = u187 ? (p < P ? u187[e * P + p] : 0.5f) : hn.get(it, lane);
         if (p < P) out_priv[r * PD + 51 + p] = hl_obs_height(c, rz, b.measured_heights[e * P + p], u);
@@ -1024,12 +1031,15 @@ __global__ void __launch_bounds__(256) hl_select_terminal_kernel(HlCfg c, HlEnvB
   unsigned* ctrl = reinterpret_cast<unsigned*>(ws);
   volatile unsigned long long* state = reinterpret_cast<volatile unsigned long long*>(ws) + 2;
   __shared__ unsigned s_vb;
+  __shared__ unsigned long long s_step;
   if (tid == 0) {   // virtual block id by ticket: a CTA only ever waits on CTAs that have already started
     s_vb = atomicAdd(ctrl, 1u);
     s_epoch = *reinterpret_cast<volatile unsigned*>(ctrl + 2) + 1u;
+    s_step = hl_step_key(b);
   }
   __syncthreads();
   const unsigned vb = s_vb;
+  const uint64_t step = s_step;
   const long long e0 = (long long)vb * SEL_ENVS;
   // one flag per thread
   const long long off = e0 + tid;
@@ -1113,7 +1123,7 @@ __global__ void __launch_bounds__(256) hl_select_terminal_kernel(HlCfg c, HlEnvB
         s.pg[k] = b.projected_gravity[e * 3 + k];
       }
       uint4 nb = make_uint4(0u, 0u, 0u, 0u);
-      if (c.add_noise && !u45) nb = hl_noise_block(b.philox_seed, b.philox_offset, (unsigned long long)s.gid, (unsigned)(cb * 32 + lane), 1u);
+      if (c.add_noise && !u45) nb = hl_noise_block(b.philox_seed, step, (unsigned long long)s.gid, (unsigned)(cb * 32 + lane), 1u);
 #pragma unroll
       for (int h = 0; h < 2; ++h) {
         const int k = lane + 32 * h;
@@ -1134,7 +1144,7 @@ __global__ void __launch_bounds__(256) hl_select_terminal_kernel(HlCfg c, HlEnvB
         for (int it = 0; it < 8; ++it) {
           if (it * 32 >= P) break;
           const int p = it * 32 + lane;
-          if (!u187 && (it & 3) == 0) hn.refill(b, (unsigned long long)s.gid, it >> 2, lane, 1u);
+          if (!u187 && (it & 3) == 0) hn.refill(b, step, (unsigned long long)s.gid, it >> 2, lane, 1u);
           float u = 0.5f;
           if (c.add_noise) u = u187 ? (p < P ? u187[e * P + p] : 0.5f) : hn.get(it, lane);
           if (p < P) out_priv[r * PD + 51 + p] = hl_obs_height(c, rz, mh[it], u);
@@ -1151,7 +1161,7 @@ __global__ void __launch_bounds__(256) hl_select_terminal_kernel(HlCfg c, HlEnvB
       if (RESET) {   // the terminal rows are out: this env may now be reset (same warp, program order)
         extern __shared__ __align__(16) float sel_stage[];
         __syncwarp();
-        hl_stage_one(c, b, rs, HL_ST_HEIGHTS | HL_ST_OBS | HL_ST_OBS_NOSHIFT | HL_ST_OBS_CLIP | HL_ST_ROLL | HL_ST_RESET_ZERO | HL_ST_RESET_DRAW,
+        hl_stage_one(c, b, step, rs, HL_ST_HEIGHTS | HL_ST_OBS | HL_ST_OBS_NOSHIFT | HL_ST_OBS_CLIP | HL_ST_ROLL | HL_ST_RESET_ZERO | HL_ST_RESET_DRAW,
                      sel_stage + wid * hl_warp_stage_floats(c.num_bodies), e, n, -1, lane, true, true, 1, 0);
         staged = false;
       }
@@ -1429,13 +1439,13 @@ struct FusedArgs {
 };
 
 // _resample_commands for the lane's env inside the fused step (same arithmetic and uniform columns as hl_resample_kernel)
-__device__ __forceinline__ void hl_fused_resample(const FusedArgs& fa, const HlEnvBuffers& b, long long ge, long long gid, float* cmd) {
+__device__ __forceinline__ void hl_fused_resample(const FusedArgs& fa, const HlEnvBuffers& b, uint64_t step, long long ge, long long gid, float* cmd) {
   float u[4];
   if (fa.rs_uniforms) {
 #pragma unroll
     for (int k = 0; k < 4; ++k) u[k] = fa.rs_uniforms[ge * HL_RESET_NU + 36 + k];
   } else {
-    const uint4 q = hl_noise_block(b.philox_seed, b.philox_offset, (unsigned long long)gid, 9u, 2u);
+    const uint4 q = hl_noise_block(b.philox_seed, step, (unsigned long long)gid, 9u, 2u);
     u[0] = hl_u01(q.x); u[1] = hl_u01(q.y); u[2] = hl_u01(q.z); u[3] = hl_u01(q.w);
   }
   float c0 = (1.0f - (-1.0f)) * u[0] + (-1.0f);

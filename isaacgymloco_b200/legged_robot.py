@@ -157,6 +157,11 @@ class FusedLeggedRobot:
         self._fused_event_hook = None      # bench.py: CUDA-event pair around the fused kernel
         self._rollout = None               # bind_rollout(): storage whose slots the env writes in place
         self._philox_bias = 0
+        # device step counter for replayed rollouts (capture_rollout): while a graph is captured the kernels key step k
+        # as *_step_base + k (_capture_base = the host counter the capture started at); None = keys by value
+        self._step_base = torch.zeros(1, dtype=torch.long, device=dev)
+        self._capture_base = None
+        self._ep_log = None                # RolloutGraph: (tables, row) the step's episode logging goes to
         self._reset_sets_physx = False
         self._prepare_terrain()
         self._init_reset_state()
@@ -218,9 +223,17 @@ class FusedLeggedRobot:
         bufs.obs_buf_out = L.ptr(self.obs_buf)
         bufs.privileged_obs_buf = L.ptr(self.privileged_obs_buf)
 
+    def _step_key(self):
+        """(philox_offset, step_base): the step index by value, or relative to the device counter while a rollout
+        graph is captured (a replay then keys its steps by the counter it finds on the device)."""
+        k = self.common_step_counter + self._philox_bias
+        if self._capture_base is None:
+            return k, None
+        return k - self._capture_base, L.ptr(self._step_base)
+
     def _buffers(self) -> L.HlEnvBuffers:
         if self._bufs is not None:
-            self._bufs.philox_offset = self.common_step_counter + self._philox_bias
+            self._bufs.philox_offset, self._bufs.step_base = self._step_key()
             return self._bufs
         b = L.HlEnvBuffers()
         b.struct_bytes = ctypes.sizeof(L.HlEnvBuffers)
@@ -246,7 +259,8 @@ class FusedLeggedRobot:
         b.obs_buf_in = b.obs_buf_out = p(self.obs_buf)
         b.privileged_obs_buf = p(self.privileged_obs_buf)
         b.noise_u45, b.noise_u187 = p(self._noise.get("obs45")), p(self._noise.get("obs187"))
-        b.philox_seed, b.philox_offset = self._philox_seed, self.common_step_counter + self._philox_bias
+        b.philox_seed = self._philox_seed
+        b.philox_offset, b.step_base = self._step_key()
         b.height_idx_out = None
         b.base_height_out = p(self._base_heights)
         if self.single_launch:
@@ -636,7 +650,8 @@ class FusedLeggedRobot:
                 if R.commands_curriculum and self.common_step_counter % self.max_episode_length == 0:   # LR:306-307 (1 step in 1000)
                     self.update_command_curriculum(self._reset_ids[:int(self._n_reset.item())])
                 r = self._reset_struct()
-                r.means_out, r.means_ws = L.ptr(self._episode_means), L.ptr(self._means_ws)
+                means = self._episode_means if self._ep_log is None else self._ep_log[0].means[self._ep_log[1]]
+                r.means_out, r.means_ws = L.ptr(means), L.ptr(self._means_ws)
                 c, b = ctypes.byref(self._c), ctypes.byref(self._buffers())
                 if push_now:
                     L.check(L.lib.hl_reset_idx(c, b, ctypes.byref(r), L.ptr(self._reset_ids), L.ptr(self._n_reset), self.num_envs, L.stream()))
@@ -651,6 +666,8 @@ class FusedLeggedRobot:
                     L.check(L.lib.hl_reset_and_fixup(c, b, ctypes.byref(r), L.ptr(self._reset_ids), L.ptr(self._n_reset), self.num_envs,
                                                      L.stream()))
                 self._reset_sets_physx = True
+                if self._ep_log is not None:
+                    self._ep_log[0].record(self, self._ep_log[1])
             else:
                 n_reset = int(self._n_reset.item())          # torch hooks need the ids on the host side (LR:225,298)
                 self.reset_idx(self._reset_ids[:n_reset])
@@ -700,6 +717,38 @@ class FusedLeggedRobot:
         self.extras["terminal_amp_states"] = term_amp
         out = (self.obs_buf, self.privileged_obs_buf, self.rew_buf, self.reset_buf, self.extras, env_ids, term_priv)
         return out + (term_amp,) if self.cfg_hot.using_amp else out
+
+    def step_device(self, actions):
+        """step() without the host sync, for CUDA-graph capture: clip, delay, `decimation` x (PD torques,
+        physics_step_fn), post_physics_step_device().  Returns (obs_buf, privileged_obs_buf, rew_buf, reset_buf, extras,
+        reset_ids, n_reset, termination_privileged_obs, terminal_amp_states): the id and terminal-row buffers have
+        capacity N and the count n_reset is a (1,) int32 device tensor (HIMRolloutStorage.record_env_step takes it as
+        termination_count).  extras["episode"] is not built here (RolloutGraph.run() returns the episode logging).
+        A live Isaac Gym sim cannot be stepped this way: gym.simulate is a host call that a graph cannot capture."""
+        if getattr(self, "gym", None) is not None:
+            raise RuntimeError("step_device() needs standalone physics (physics_step_fn): gym.simulate cannot be captured")
+        clip = self.cfg_hot.clip_actions
+        torch.clamp(actions.to(self.device), -clip, clip, out=self.actions)
+        self._delay_actions()
+        for k in range(self.cfg_hot.decimation):
+            self._compute_torques_into(self.delayed_actions[:, k], self.torques)
+            if self.physics_step_fn is not None:
+                self.physics_step_fn(self, k)
+        ids, n_dev, term_priv, term_amp = self.post_physics_step_device()
+        self.extras["time_outs"] = self.time_out_buf
+        self.extras["terminal_amp_states"] = term_amp
+        return (self.obs_buf, self.privileged_obs_buf, self.rew_buf, self.reset_buf, self.extras, ids, n_dev, term_priv,
+                term_amp)
+
+    def capture_rollout(self, body: Callable[[int], None], num_steps: int, storage=None, finish: Optional[Callable[[], None]] = None,
+                        max_graphs: int = 8, warmup: int = 1):
+        """A RolloutGraph that runs `body(0) .. body(num_steps - 1)` then `finish()` as one captured CUDA graph whenever
+        the rollout window allows it, and eagerly otherwise (rollout_graph.py).  `body(k)` is the runner's per-step
+        code (act -> step_device -> storage.record_env_step(..., termination_count=n_reset)); `finish` e.g.
+        compute_returns; `storage`: the HIMRolloutStorage the body records into.  `max_graphs` bounds the cache of
+        captured graphs; the first `warmup` rollouts run eagerly."""
+        from .rollout_graph import RolloutGraph
+        return RolloutGraph(self, body, num_steps, storage=storage, finish=finish, max_graphs=max_graphs, warmup=warmup)
 
     # ------------------------------------------------------------------ torch-side hooks (RNG / PhysX)
     def _delay_actions(self):
