@@ -323,6 +323,13 @@ typedef struct HlReset {
    * doubles, zeroed ONCE at allocation (the kernel re-arms it). */
   float* means_out;                /* (n_rows,) or NULL */
   double* means_ws;
+  /* (8,) device float64 command ranges in the order of the by-value fields (lin_vel_x lo,hi | lin_vel_y lo,hi |
+   * ang_vel_yaw lo,hi | heading lo,hi) or NULL = the by-value cmd_* fields.  Set: every command draw (hl_resample_commands,
+   * the re-draws of the reset launches, the fused step's pre-step resampling through resample_host) reads the ranges
+   * here, after griddepcontrol.wait, and converts each with (float) -- the round-to-nearest a c_float assignment of the
+   * same Python float does, so both forms draw bit-identical commands from equal values.  A captured graph then follows
+   * range changes made on the device (hl_command_curriculum) or copied there between replays. */
+  const double* cmd_ranges;
 } HlReset;
 int hl_sizeof_reset(void);
 /* reset_idx(env_ids) without the fix-up: curriculum, state re-draws, the RNG-free buffer resets (LR:323-329,361). */
@@ -340,6 +347,16 @@ int hl_reset_and_fixup(const HlCfg* cfg, const HlEnvBuffers* bufs, const HlReset
  * increments the counter.  Uniform columns 36-39 (Philox stream 2 for the pre-step form). */
 int hl_resample_commands(const HlCfg* cfg, const HlEnvBuffers* bufs, const HlReset* reset, const int64_t* env_ids,
                          const int32_t* n_ids_dev, int64_t interval, int64_t n_envs, void* stream);
+/* update_command_curriculum(env_ids) (LR:868-880) on device-resident ranges, as one capturable launch (one CTA, no host
+ * sync, no allocation).  n = *n_ids_dev; n == 0 leaves the ranges alone.  Otherwise s = float64 sum of
+ * tracking_sums[env_ids[i]], v = fp32(fp32(s / n) / fp32(max_episode_length)), and when (double)v > threshold the
+ * lin_vel_x / lin_vel_y bounds move by -+0.1 and are clipped in float64 as np.clip does: x lo to [-max_backward, 0],
+ * x hi to [0, max_forward], y lo to [-max_lat, 0], y hi to [0, max_lat].  ranges: (8,) in/out, HlReset.cmd_ranges order;
+ * ranges_log: (8,) or NULL, receives the ranges after the decision.  The host's fp32 torch.mean sums in another order, so
+ * the two decisions can differ when the mean lies within a few ulp of the threshold. */
+int hl_command_curriculum(const float* tracking_sums, const int64_t* env_ids, const int32_t* n_ids_dev, double threshold,
+                          int64_t max_episode_length, double max_backward, double max_forward, double max_lat,
+                          double* ranges, double* ranges_log, int64_t n_envs, void* stream);
 
 /* ReplayBuffer.insert(states, next_states) -- rsl_rl/rsl_rl/storage/replay_buffer.py:52-68: row r of
  * both (n_rows, width) inputs is written to ring row (step + r) mod buffer_rows; when more than

@@ -83,6 +83,7 @@ EXPORTS = {
     "hl_reset_draw": (c_int32, [POINTER(HlCfg), POINTER(HlEnvBuffers), POINTER(HlReset), _vp, _vp, c_int64, _vp]),
     "hl_reset_and_fixup": (c_int32, [POINTER(HlCfg), POINTER(HlEnvBuffers), POINTER(HlReset), _vp, _vp, c_int64, _vp]),
     "hl_resample_commands": (c_int32, [POINTER(HlCfg), POINTER(HlEnvBuffers), POINTER(HlReset), _vp, _vp, c_int64, c_int64, _vp]),
+    "hl_command_curriculum": (c_int32, [_vp, _vp, _vp, c_double, c_int64, c_double, c_double, c_double, _vp, _vp, c_int64, _vp]),
     "hl_episode_means": (c_int32, [_vp, _vp, _vp, _vp, c_int32, c_int64, c_float, c_int32, _vp, _vp]),
     "hl_amp_observations": (c_int32, [_vp, _vp, _vp, _vp, c_int64, _vp]),
     "hl_gae_scan": (c_int32, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, c_int32, c_int64, c_float, c_float, _vp]),

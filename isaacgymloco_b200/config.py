@@ -147,7 +147,7 @@ class HlReset(ctypes.Structure):
         ("cmd_heading", ctypes.c_float * 2), ("env_length", ctypes.c_float),
         ("max_episode_length_s", ctypes.c_float)] + [(n, ctypes.c_void_p) for n in (
         "root_states", "dof_state", "commands", "env_origins", "terrain_origins", "terrain_levels", "terrain_types",
-        "kp_factors", "kd_factors", "motor_strength_factors", "uniforms", "means_out", "means_ws")]
+        "kp_factors", "kd_factors", "motor_strength_factors", "uniforms", "means_out", "means_ws", "cmd_ranges")]
 
 
 def high_vel_env_count(num_envs: int) -> int:

@@ -403,12 +403,28 @@ struct ResetUniforms {
   }
 };
 
-// _resample_commands for one env (LR:634-656); lane 0 stores
-__device__ __forceinline__ void hl_resample_env(const HlReset& r, const ResetUniforms& ru, long long e, long long gid, int lane) {
+// The command ranges of a HlReset as 8 floats (lin_vel_x, lin_vel_y, ang_vel_yaw, heading; lo, hi) in `slot` (shared
+// memory): from the device copy when reset.cmd_ranges is set (read after griddepcontrol.wait), else the by-value fields.
+// Thread 0 stores; the caller's next __syncthreads publishes them to the CTA.
+__device__ __forceinline__ void hl_cmd_ranges_cta(const HlReset& r, float* slot) {
+  if (threadIdx.x != 0) return;
+  if (r.cmd_ranges) {
+#pragma unroll
+    for (int k = 0; k < 8; ++k) slot[k] = (float)r.cmd_ranges[k];
+  } else {
+    slot[0] = r.cmd_lin_vel_x[0]; slot[1] = r.cmd_lin_vel_x[1];
+    slot[2] = r.cmd_lin_vel_y[0]; slot[3] = r.cmd_lin_vel_y[1];
+    slot[4] = r.cmd_ang_vel_yaw[0]; slot[5] = r.cmd_ang_vel_yaw[1];
+    slot[6] = r.cmd_heading[0]; slot[7] = r.cmd_heading[1];
+  }
+}
+
+// _resample_commands for one env (LR:634-656); lane 0 stores.  cr: the CTA's command ranges (hl_cmd_ranges_cta)
+__device__ __forceinline__ void hl_resample_env(const HlReset& r, const float* cr, const ResetUniforms& ru, long long e, long long gid, int lane) {
   float c0 = (1.0f - (-1.0f)) * ru.get(36) + (-1.0f);            // LR:641
-  float c1 = ru.range(37, r.cmd_lin_vel_y);                        // LR:642
-  const float c3 = ru.range(38, r.heading_command ? r.cmd_heading : r.cmd_ang_vel_yaw);   // LR:643-646
-  const float hv = ru.range(39, r.cmd_lin_vel_x);
+  float c1 = ru.range(37, cr + 2);                                 // LR:642
+  const float c3 = ru.range(38, r.heading_command ? cr + 6 : cr + 4);   // LR:643-646
+  const float hv = ru.range(39, cr);
   if (gid < r.high_vel_envs) {   // LR:649-653 (env_ids < num_envs * 0.2)
     c0 = hv;
     c1 *= fabsf(c0) < 1.0f ? 1.0f : 0.0f;     // norm of a 1-vector
@@ -425,7 +441,8 @@ __device__ __forceinline__ void hl_resample_env(const HlReset& r, const ResetUni
 
 // reset_idx for env e, the part that draws: terrain curriculum, dofs, root state, commands, gain factors
 // (LR:301-320,336-341).  Warp-cooperative: lanes 0-11 own one dof each, lane 0 the scalars.
-__device__ __forceinline__ void hl_reset_draw_env(const HlCfg& c, const HlEnvBuffers& b, uint64_t step, const HlReset& r, long long e, int lane) {
+__device__ __forceinline__ void hl_reset_draw_env(const HlCfg& c, const HlEnvBuffers& b, uint64_t step, const HlReset& r, const float* cr,
+                                                  long long e, int lane) {
   const long long gid = e + c.env_id_offset;
   ResetUniforms ru;
   ru.init(b, step, r, e, (unsigned long long)gid, lane, 3u);
@@ -508,7 +525,7 @@ __device__ __forceinline__ void hl_reset_draw_env(const HlCfg& c, const HlEnvBuf
     if (lane < 6) r.root_states[e * 13 + 7 + lane] = vel6;
   }
   // ---- _resample_commands (LR:634-656)
-  if (parts & HL_RESET_COMMANDS) hl_resample_env(r, ru, e, gid, lane);
+  if (parts & HL_RESET_COMMANDS) hl_resample_env(r, cr, ru, e, gid, lane);
   // ---- Kp / Kd / motor-strength factors (LR:336-341)
   if (parts & HL_RESET_FACTORS) {
     const float ukp = ru.get(40), ukd = ru.get(41), ums = ru.get(42);
@@ -526,14 +543,15 @@ __device__ __forceinline__ void hl_reset_draw_env(const HlCfg& c, const HlEnvBuf
 // buffer resets, slot 0 / privileged_obs[0:51] and the roll, the others the height iterations it % it_mod == it_rem).
 // `items`: length of the id list -- the warp that completes it finalises the episode-logging means; < 0 = the caller
 // finalises them itself.  `st`: this warp's staging area (hl_warp_stage_floats floats of shared memory).  `step`: the Philox step key.
-__device__ __forceinline__ void hl_stage_one(const HlCfg& c, const HlEnvBuffers& b, const uint64_t step, const HlReset& rs, const unsigned stages, float* st,
-                                             const long long e, const long long n, const long long items, const int lane,
-                                             const bool lead, const bool scans, const int it_mod, const int it_rem) {
+// `cr`: the CTA's command ranges (hl_cmd_ranges_cta; read with HL_ST_RESET_DRAW only).
+__device__ __forceinline__ void hl_stage_one(const HlCfg& c, const HlEnvBuffers& b, const uint64_t step, const HlReset& rs, const float* cr,
+                                             const unsigned stages, float* st, const long long e, const long long n, const long long items,
+                                             const int lane, const bool lead, const bool scans, const int it_mod, const int it_rem) {
   const int B = c.num_bodies;
   const int P = c.n_px * c.n_py;
   const int PD = hl_priv_dim(c);
   __syncwarp();   // the previous env's staged records are no longer read
-  if ((stages & HL_ST_RESET_DRAW) && lead) hl_reset_draw_env(c, b, step, rs, e, lane);   // writes the env's root / dof / command rows
+  if ((stages & HL_ST_RESET_DRAW) && lead) hl_reset_draw_env(c, b, step, rs, cr, e, lane);   // writes the env's root / dof / command rows
   EnvView v;
   hl_stage_env(st, c, b, e, lane, (stages & HL_ST_RESET_ZERO) != 0, v);
   if ((stages & HL_ST_RESET_ZERO) && lead) {  // LR:323-329,350,361
@@ -756,9 +774,11 @@ __global__ void __launch_bounds__(256, 3) hl_stage_kernel(HlCfg c, HlEnvBuffers 
   // it % (parts-1) == part-1 (scan + height part of privileged_obs): shorter dependent chains for the
   // few hundred reset envs of a step.
   hl_pdl_enter();
-  __shared__ unsigned long long s_step;
-  const uint64_t step = hl_step_key_cta(b, &s_step);
   const unsigned stages = STAGES ? STAGES : stages_rt;
+  __shared__ unsigned long long s_step;
+  __shared__ float s_cr[8];
+  if (stages & HL_ST_RESET_DRAW) hl_cmd_ranges_cta(rs, s_cr);   // published by hl_step_key_cta's barrier
+  const uint64_t step = hl_step_key_cta(b, &s_step);
   const int lane = threadIdx.x & 31;
   const long long warp0 = ((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
   const long long nwarps = ((long long)gridDim.x * blockDim.x) >> 5;
@@ -774,7 +794,7 @@ __global__ void __launch_bounds__(256, 3) hl_stage_kernel(HlCfg c, HlEnvBuffers 
     const int it_mod = np == 1 ? 1 : np - 1, it_rem = np == 1 ? 0 : part - 1;
     const long long e = ids ? ids[it0] : it0;
     if (e < 0 || e >= n) continue;
-    hl_stage_one(c, b, step, rs, stages, st, e, n, items, lane, lead, scans, it_mod, it_rem);
+    hl_stage_one(c, b, step, rs, s_cr, stages, st, e, n, items, lane, lead, scans, it_mod, it_rem);
   }
 }
 
@@ -858,6 +878,8 @@ __global__ void __launch_bounds__(256) hl_resample_kernel(HlCfg c, HlEnvBuffers 
                                                           const int* __restrict__ n_ids, long long interval, long long n) {
   hl_pdl_enter();
   __shared__ unsigned long long s_step;
+  __shared__ float cr[8];
+  hl_cmd_ranges_cta(r, cr);                               // published by hl_step_key_cta's barrier
   const uint64_t step = hl_step_key_cta(b, &s_step);
   const long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   long long e;
@@ -880,11 +902,11 @@ __global__ void __launch_bounds__(256) hl_resample_kernel(HlCfg c, HlEnvBuffers 
     u[0] = hl_u01(q.x); u[1] = hl_u01(q.y); u[2] = hl_u01(q.z); u[3] = hl_u01(q.w);
   }
   float c0 = (1.0f - (-1.0f)) * u[0] + (-1.0f);
-  float c1 = (r.cmd_lin_vel_y[1] - r.cmd_lin_vel_y[0]) * u[1] + r.cmd_lin_vel_y[0];
-  const float* lohi = r.heading_command ? r.cmd_heading : r.cmd_ang_vel_yaw;
+  float c1 = (cr[3] - cr[2]) * u[1] + cr[2];
+  const float* lohi = r.heading_command ? cr + 6 : cr + 4;
   const float c3 = (lohi[1] - lohi[0]) * u[2] + lohi[0];
   if (gid < r.high_vel_envs) {
-    c0 = (r.cmd_lin_vel_x[1] - r.cmd_lin_vel_x[0]) * u[3] + r.cmd_lin_vel_x[0];
+    c0 = (cr[1] - cr[0]) * u[3] + cr[0];
     c1 *= fabsf(c0) < 1.0f ? 1.0f : 0.0f;
   }
   const float keep = sqrtf(c0 * c0 + c1 * c1) > 0.2f ? 1.0f : 0.0f;
@@ -902,6 +924,52 @@ extern "C" int hl_resample_commands(const HlCfg* cfg, const HlEnvBuffers* bufs, 
   if (n <= 0) return HL_OK;
   hl_launch(hl_resample_kernel, dim3((unsigned)((n + 255) / 256)), dim3(256), 0, (cudaStream_t)stream, *cfg, *bufs, *reset,
             (const long long*)env_ids, n_ids_dev, (long long)interval, (long long)n);
+  HL_CHECK_LAUNCH();
+  return HL_OK;
+}
+
+// update_command_curriculum (LR:868-880) on the device ranges: one CTA, a grid-stride float64 sum over the reset ids, then
+// thread 0 decides and moves the ranges.  It runs once per max_episode_length steps: a multi-CTA reduction is not worth it.
+__global__ void __launch_bounds__(256) hl_command_curriculum_kernel(const float* __restrict__ sums, const long long* __restrict__ ids,
+                                                                    const int* __restrict__ n_ids, double threshold, long long max_len,
+                                                                    double max_backward, double max_forward, double max_lat,
+                                                                    double* ranges, double* ranges_log, long long n) {
+  hl_pdl_enter();
+  __shared__ double part[8];
+  const int tid = threadIdx.x;
+  const long long cnt = *n_ids;
+  double s = 0.0;
+  for (long long i = tid; i < cnt; i += blockDim.x) {
+    const long long e = ids[i];
+    if (e >= 0 && e < n) s += (double)sums[e];
+  }
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
+  if ((tid & 31) == 0) part[tid >> 5] = s;
+  __syncthreads();
+  if (tid != 0) return;
+  double tot = 0.0;
+  for (int w = 0; w < (int)(blockDim.x >> 5); ++w) tot += part[w];
+  if (cnt > 0) {   // the host returns early on an empty id list
+    const float v = __fdiv_rn((float)(tot / (double)cnt), (float)max_len);   // fp32 mean, then the fp32 divide by the length
+    if ((double)v > threshold) {   // np.clip(x, lo, hi) == min(max(x, lo), hi), in float64
+      ranges[0] = fmin(fmax(ranges[0] - 0.1, -max_backward), 0.0);
+      ranges[1] = fmin(fmax(ranges[1] + 0.1, 0.0), max_forward);
+      ranges[2] = fmin(fmax(ranges[2] - 0.1, -max_lat), 0.0);
+      ranges[3] = fmin(fmax(ranges[3] + 0.1, 0.0), max_lat);
+    }
+  }
+  if (ranges_log)
+    for (int k = 0; k < 8; ++k) ranges_log[k] = ranges[k];
+}
+
+extern "C" int hl_command_curriculum(const float* tracking_sums, const int64_t* env_ids, const int32_t* n_ids_dev, double threshold,
+                                     int64_t max_episode_length, double max_backward, double max_forward, double max_lat,
+                                     double* ranges, double* ranges_log, int64_t n, void* stream) {
+  HL_CHECK_ARG(tracking_sums && env_ids && n_ids_dev && ranges, "null pointer");
+  HL_CHECK_ARG(max_episode_length > 0, "max_episode_length must be positive");
+  hl_launch(hl_command_curriculum_kernel, dim3(1), dim3(256), 0, (cudaStream_t)stream, tracking_sums, (const long long*)env_ids,
+            n_ids_dev, threshold, (long long)max_episode_length, max_backward, max_forward, max_lat, ranges, ranges_log, (long long)n);
   HL_CHECK_LAUNCH();
   return HL_OK;
 }
@@ -1032,11 +1100,13 @@ __global__ void __launch_bounds__(256) hl_select_terminal_kernel(HlCfg c, HlEnvB
   volatile unsigned long long* state = reinterpret_cast<volatile unsigned long long*>(ws) + 2;
   __shared__ unsigned s_vb;
   __shared__ unsigned long long s_step;
+  __shared__ float s_cr[8];
   if (tid == 0) {   // virtual block id by ticket: a CTA only ever waits on CTAs that have already started
     s_vb = atomicAdd(ctrl, 1u);
     s_epoch = *reinterpret_cast<volatile unsigned*>(ctrl + 2) + 1u;
     s_step = hl_step_key(b);
   }
+  if (RESET) hl_cmd_ranges_cta(rs, s_cr);
   __syncthreads();
   const unsigned vb = s_vb;
   const uint64_t step = s_step;
@@ -1161,7 +1231,7 @@ __global__ void __launch_bounds__(256) hl_select_terminal_kernel(HlCfg c, HlEnvB
       if (RESET) {   // the terminal rows are out: this env may now be reset (same warp, program order)
         extern __shared__ __align__(16) float sel_stage[];
         __syncwarp();
-        hl_stage_one(c, b, step, rs, HL_ST_HEIGHTS | HL_ST_OBS | HL_ST_OBS_NOSHIFT | HL_ST_OBS_CLIP | HL_ST_ROLL | HL_ST_RESET_ZERO | HL_ST_RESET_DRAW,
+        hl_stage_one(c, b, step, rs, s_cr, HL_ST_HEIGHTS | HL_ST_OBS | HL_ST_OBS_NOSHIFT | HL_ST_OBS_CLIP | HL_ST_ROLL | HL_ST_RESET_ZERO | HL_ST_RESET_DRAW,
                      sel_stage + wid * hl_warp_stage_floats(c.num_bodies), e, n, -1, lane, true, true, 1, 0);
         staged = false;
       }
@@ -1430,6 +1500,7 @@ struct FusedArgs {
   long long rs_hi_envs;   // HlReset::high_vel_envs (LR:649)
   float rs_lin_vel_x[2], rs_lin_vel_y[2], rs_third[2];   // third = heading range (heading_command) or yaw-rate range
   const float* rs_uniforms;   // (N, HL_RESET_NU) or nullptr => Philox stream 2
+  const double* rs_ranges;    // HlReset::cmd_ranges (device) or nullptr => the by-value rs_* ranges above
   int hist_pf;            // bulk-prefetch the tile's obs-history slab into L2 (obs_buf_in 16-B aligned)
   int tma_ok;             // every dense slab of a full tile is 16-B aligned with a 16-B multiple size (n % 4 == 0, aligned bases)
   int sums_aligned;       // episode_sums rows are 16-B aligned per block (n % 4 == 0, base aligned)
@@ -1448,11 +1519,19 @@ __device__ __forceinline__ void hl_fused_resample(const FusedArgs& fa, const HlE
     const uint4 q = hl_noise_block(b.philox_seed, step, (unsigned long long)gid, 9u, 2u);
     u[0] = hl_u01(q.x); u[1] = hl_u01(q.y); u[2] = hl_u01(q.z); u[3] = hl_u01(q.w);
   }
+  // the ranges: by value, or from the device copy (this branch runs after the kernel's griddepcontrol.wait)
+  float x0 = fa.rs_lin_vel_x[0], x1 = fa.rs_lin_vel_x[1], y0 = fa.rs_lin_vel_y[0], y1 = fa.rs_lin_vel_y[1], t0 = fa.rs_third[0],
+        t1 = fa.rs_third[1];
+  if (fa.rs_ranges) {
+    const double* q = fa.rs_ranges;
+    const int o = fa.rs_heading ? 6 : 4;
+    x0 = (float)q[0]; x1 = (float)q[1]; y0 = (float)q[2]; y1 = (float)q[3]; t0 = (float)q[o]; t1 = (float)q[o + 1];
+  }
   float c0 = (1.0f - (-1.0f)) * u[0] + (-1.0f);
-  float c1 = (fa.rs_lin_vel_y[1] - fa.rs_lin_vel_y[0]) * u[1] + fa.rs_lin_vel_y[0];
-  const float c3 = (fa.rs_third[1] - fa.rs_third[0]) * u[2] + fa.rs_third[0];
+  float c1 = (y1 - y0) * u[1] + y0;
+  const float c3 = (t1 - t0) * u[2] + t0;
   if (gid < fa.rs_hi_envs) {
-    c0 = (fa.rs_lin_vel_x[1] - fa.rs_lin_vel_x[0]) * u[3] + fa.rs_lin_vel_x[0];
+    c0 = (x1 - x0) * u[3] + x0;
     c1 *= fabsf(c0) < 1.0f ? 1.0f : 0.0f;
   }
   const float keep = sqrtf(c0 * c0 + c1 * c1) > 0.2f ? 1.0f : 0.0f;
@@ -1587,6 +1666,7 @@ extern "C" int hl_post_physics_fused(const HlCfg* cfg, const HlEnvBuffers* bufs,
     fa.tma_ok = ok;
     fa.rs_interval = 0;
     fa.rs_uniforms = nullptr;
+    fa.rs_ranges = nullptr;
     if (b.resample_host && b.resample_interval > 0) {
       const HlReset* r = b.resample_host;
       HL_CHECK_ARG(r->struct_bytes == (int)sizeof(HlReset), "resample_host: HlReset size mismatch");
@@ -1598,6 +1678,7 @@ extern "C" int hl_post_physics_fused(const HlCfg* cfg, const HlEnvBuffers* bufs,
       const float* third = r->heading_command ? r->cmd_heading : r->cmd_ang_vel_yaw;
       fa.rs_third[0] = third[0]; fa.rs_third[1] = third[1];
       fa.rs_uniforms = r->uniforms;
+      fa.rs_ranges = r->cmd_ranges;
     }
     const char* pf = getenv("HL_PK_HIST_PF");   // experiment knob
     fa.hist_pf = (((uintptr_t)b.obs_buf_in & 15) == 0) && !(pf && pf[0] == '0');

@@ -411,6 +411,11 @@ class FusedLeggedRobot:
                                        ang_vel_yaw=list(R.ang_vel_yaw), heading=list(R.heading))
         if not hasattr(self, "init_done"):
             self.init_done = True
+        # device copy of command_ranges (HlReset.cmd_ranges order), read by the kernels only in the device-schedule mode of
+        # RolloutGraph.run(); _cmd_ranges_mirror = the host values it holds (None = not uploaded yet)
+        self._cmd_ranges_dev = z(8, dtype=torch.float64)
+        self._cmd_ranges_mirror = None
+        self._device_schedule = False
         self._high_vel_envs = high_vel_env_count(self.cfg_hot.num_envs)         # LR:649, keyed by the global env id
         self._reset_uniforms = None           # parity mode: (N, RESET_NU) pre-drawn U[0,1)
         self._episode_means = z(max(self._episode_sums_buf.shape[0], 1))
@@ -450,9 +455,14 @@ class FusedLeggedRobot:
         r.randomize_kp, r.randomize_kd, r.randomize_motor_strength = int(R.randomize_kp), int(R.randomize_kd), int(R.randomize_motor_strength)
         r.kp_range[:], r.kd_range[:], r.motor_strength_range[:] = R.kp_range, R.kd_range, R.motor_strength_range
         r.heading_command = int(self.cfg_hot.heading_command)
-        cr = self.command_ranges
-        r.cmd_lin_vel_x[:], r.cmd_lin_vel_y[:] = cr["lin_vel_x"], cr["lin_vel_y"]
-        r.cmd_ang_vel_yaw[:], r.cmd_heading[:] = cr["ang_vel_yaw"], cr["heading"]
+        if self._device_schedule:
+            # the kernels read the device copy; the by-value fields stay zero, so a captured graph's signature does not
+            # change when the curriculum or the user moves the ranges
+            r.cmd_ranges = L.ptr(self._cmd_ranges_dev)
+        else:
+            cr = self.command_ranges
+            r.cmd_lin_vel_x[:], r.cmd_lin_vel_y[:] = cr["lin_vel_x"], cr["lin_vel_y"]
+            r.cmd_ang_vel_yaw[:], r.cmd_heading[:] = cr["ang_vel_yaw"], cr["heading"]
         r.num_envs_global = self.cfg_hot.num_envs
         r.high_vel_envs = self._high_vel_envs
         has_cur = R.terrain_curriculum and self.init_done and self.terrain_origins is not None and self.terrain_types is not None
@@ -566,6 +576,43 @@ class FusedLeggedRobot:
             cr["lin_vel_y"][0] = float(np.clip(cr["lin_vel_y"][0] - 0.1, -getattr(R, "max_lat_curriculum", 1.0), 0.))
             cr["lin_vel_y"][1] = float(np.clip(cr["lin_vel_y"][1] + 0.1, 0., getattr(R, "max_lat_curriculum", 1.0)))
 
+    # ------------------------------------------------------------------ device-resident command ranges
+    COMMAND_RANGE_KEYS = ("lin_vel_x", "lin_vel_y", "ang_vel_yaw", "heading")
+
+    def command_ranges_flat(self):
+        """command_ranges as the 8 floats of HlReset.cmd_ranges (lo, hi of lin_vel_x, lin_vel_y, ang_vel_yaw, heading)."""
+        return tuple(float(self.command_ranges[k][j]) for k in self.COMMAND_RANGE_KEYS for j in (0, 1))
+
+    def set_command_ranges_flat(self, vals):
+        """Write 8 floats into command_ranges, in place (the lists keep their identity)."""
+        for i, k in enumerate(self.COMMAND_RANGE_KEYS):
+            self.command_ranges[k][0], self.command_ranges[k][1] = float(vals[2 * i]), float(vals[2 * i + 1])
+
+    def _upload_command_ranges(self):
+        """Copy command_ranges to the device copy when they differ from what it holds (a host edit, or the first use)."""
+        host = self.command_ranges_flat()
+        if host != self._cmd_ranges_mirror:
+            self._cmd_ranges_dev.copy_(torch.tensor(host, dtype=torch.float64))
+            self._cmd_ranges_mirror = host
+
+    def _device_curriculum_ok(self) -> bool:
+        """The command curriculum can run on the device: update_command_curriculum is not overridden."""
+        return type(self).update_command_curriculum is FusedLeggedRobot.update_command_curriculum
+
+    def _command_curriculum_device(self, ranges_log=None):
+        """update_command_curriculum(reset ids) on the device copy of the ranges: one launch, no host sync
+        (hl_command_curriculum; its float64 sum can decide differently from torch's fp32 mean only within a few ulp of
+        the threshold).  ranges_log: an (8,) float64 row that receives the ranges after the decision, or None."""
+        if "tracking_lin_vel" not in self.episode_sums:
+            return
+        R = self.cfg_hot.reset
+        L.check(L.lib.hl_command_curriculum(
+            L.ptr(self.episode_sums["tracking_lin_vel"]), L.ptr(self._reset_ids), L.ptr(self._n_reset),
+            0.8 * self.reward_scales["tracking_lin_vel"], int(self.max_episode_length),
+            float(getattr(R, "max_backward_curriculum", 1.0)), float(getattr(R, "max_forward_curriculum", 1.5)),
+            float(getattr(R, "max_lat_curriculum", 1.0)), L.ptr(self._cmd_ranges_dev), L.ptr(ranges_log), self.num_envs,
+            L.stream()))
+
     def _pre_step_callbacks(self, resample_in_fused=False):
         """The RNG-driven part of _post_physics_step_callback that precedes the fused step (LR:612-613,631-632):
         commands of the envs whose incremented episode length hits the resampling interval (in-kernel, Philox
@@ -631,6 +678,8 @@ class FusedLeggedRobot:
             if push_now:
                 # LR:627-628: the push changes root_states[:, 7:9] AFTER base_lin_vel was taken and BEFORE rewards /
                 # observations: the staged path splits the step around it (1 step in push_interval)
+                if getattr(self, "_rollout", None) is not None:
+                    self._bind_rollout_slot(self._buffers())   # read slot step, write slot step+1, as the fused path does
                 self._stages(L.ST_COUNTERS | L.ST_FRAME | L.ST_CONTACTS)
                 self._push_robots()
                 self._stages(L.ST_HEADING | L.ST_HEIGHTS | L.ST_TERMINATION | L.ST_REWARD)
@@ -648,7 +697,11 @@ class FusedLeggedRobot:
                 self.fused_pre_reset(select=not merged)
             if self._kernel_reset_ok():
                 if R.commands_curriculum and self.common_step_counter % self.max_episode_length == 0:   # LR:306-307 (1 step in 1000)
-                    self.update_command_curriculum(self._reset_ids[:int(self._n_reset.item())])
+                    if self._device_schedule and self._device_curriculum_ok():
+                        log = None if self._ep_log is None else self._ep_log[0].ranges_log[self._ep_log[1]]
+                        self._command_curriculum_device(log)
+                    else:
+                        self.update_command_curriculum(self._reset_ids[:int(self._n_reset.item())])
                 r = self._reset_struct()
                 means = self._episode_means if self._ep_log is None else self._ep_log[0].means[self._ep_log[1]]
                 r.means_out, r.means_ws = L.ptr(means), L.ptr(self._means_ws)
@@ -741,14 +794,17 @@ class FusedLeggedRobot:
                 term_amp)
 
     def capture_rollout(self, body: Callable[[int], None], num_steps: int, storage=None, finish: Optional[Callable[[], None]] = None,
-                        max_graphs: int = 8, warmup: int = 1):
+                        max_graphs: int = 8, warmup: int = 1, capture_schedule: bool = False):
         """A RolloutGraph that runs `body(0) .. body(num_steps - 1)` then `finish()` as one captured CUDA graph whenever
         the rollout window allows it, and eagerly otherwise (rollout_graph.py).  `body(k)` is the runner's per-step
         code (act -> step_device -> storage.record_env_step(..., termination_count=n_reset)); `finish` e.g.
         compute_returns; `storage`: the HIMRolloutStorage the body records into.  `max_graphs` bounds the cache of
-        captured graphs; the first `warmup` rollouts run eagerly."""
+        captured graphs; the first `warmup` rollouts run eagerly.  `capture_schedule=True` also replays windows with
+        push and command-curriculum steps: inside run() the command ranges live on the device and the curriculum
+        decides there (its float64 sum can differ from the host's fp32 mean within a few ulp of the threshold)."""
         from .rollout_graph import RolloutGraph
-        return RolloutGraph(self, body, num_steps, storage=storage, finish=finish, max_graphs=max_graphs, warmup=warmup)
+        return RolloutGraph(self, body, num_steps, storage=storage, finish=finish, max_graphs=max_graphs, warmup=warmup,
+                            capture_schedule=capture_schedule)
 
     # ------------------------------------------------------------------ torch-side hooks (RNG / PhysX)
     def _delay_actions(self):

@@ -11,7 +11,9 @@ rollout run eagerly:
   `push_interval` steps (the staged path), the command curriculum every `max_episode_length` steps (an .item()) --
   and everything copied into the launches (command and reset ranges) are frozen in a graph.  `rollout_window()`
   decides per window whether a captured graph fits; `RolloutGraph.run()` replays one when it does and runs the same
-  `body` eagerly when it does not.
+  `body` eagerly when it does not.  With capture_schedule=True the push step (staged launches + torch RNG, no host
+  sync) is captured as is, and the command ranges and the curriculum decision move to the device (HlReset.cmd_ranges,
+  hl_command_curriculum), so windows with either step replay too; graphs are then cached by all three step positions.
 
 torch-RNG hooks inside `body` (_delay_actions, _disturbance_robots, the policy's action sampling) stay torch: PyTorch's
 graph-safe Philox gives them fresh draws on every replay.  A live Isaac Gym sim cannot be captured (gym.simulate is
@@ -30,15 +32,21 @@ def _first_multiple(lo: int, m: int) -> int:
 
 
 def rollout_window(counter: int, num_steps: int, disturbance_interval: int = 0, push_interval: int = 0,
-                   curriculum_interval: int = 0) -> Tuple[Optional[Tuple[int, ...]], Optional[str]]:
+                   curriculum_interval: int = 0, in_graph: bool = False) -> Tuple[Optional[tuple], Optional[str]]:
     """Can the `num_steps` env steps that start at common_step_counter `counter` replay a captured graph?
 
     Step k of the window runs with the counter at counter + k + 1 (post_physics_step increments it first) and the
     host decides on that value: a disturbance when it is a multiple of `disturbance_interval`, a push when it is a
     multiple of `push_interval`, the command curriculum when it is a multiple of `curriculum_interval`; 0 = never.
     Returns (key, None), key = the window's steps k that apply a disturbance (graphs are cached by it), or
-    (None, reason) when the window has to run eagerly."""
+    (None, reason) when the window has to run eagerly.
+
+    in_graph=True (push and curriculum steps captured too, RolloutGraph(capture_schedule=True)): every window
+    replays, and key = (disturbance steps, push steps, curriculum steps)."""
     lo, hi = counter + 1, counter + num_steps
+    if in_graph:
+        at = lambda m: tuple(range(_first_multiple(lo, m) - lo, num_steps, m)) if m > 0 else ()
+        return (at(disturbance_interval), at(push_interval), at(curriculum_interval)), None
     for name, m in (("push", push_interval), ("command-curriculum", curriculum_interval)):
         if m > 0 and _first_multiple(lo, m) <= hi:
             return None, f"{name} step at counter {_first_multiple(lo, m)}"
@@ -56,6 +64,18 @@ def env_schedule(env) -> Dict[str, int]:
                 curriculum_interval=int(env.max_episode_length) if R.commands_curriculum else 0)
 
 
+def max_command_x_per_step(start: float, curriculum_steps, logged_rows, num_steps: int) -> List[float]:
+    """The per-step max_command_x of a rollout whose curriculum ran on the device: the value at the start of the rollout,
+    carried forward and switched at each curriculum step k to lin_vel_x[1] of the ranges that step logged (row k of
+    `logged_rows`, HlReset.cmd_ranges order)."""
+    steps, cur, out = set(curriculum_steps), float(start), []
+    for k in range(num_steps):
+        if k in steps:
+            cur = float(logged_rows[k][1])
+        out.append(cur)
+    return out
+
+
 class EpisodeTables:
     """reset_idx's episode logging (LR:344-359) of every step of one rollout, kept on the device so the rollout needs
     no host sync: the reset launch of step k writes its means to row k (HlReset.means_out), and the step adds its reset
@@ -67,9 +87,13 @@ class EpisodeTables:
         self.counts = torch.zeros(num_steps, dtype=torch.int32, device=dev)
         self.terrain_sum = torch.zeros(num_steps, dtype=torch.long, device=dev)
         self.max_command_x = [0.0] * num_steps
+        # device-schedule mode: row k = the command ranges after the curriculum decision of step k (written by that
+        # step's hl_command_curriculum launch only), and the device ranges after the rollout
+        self.ranges_log = torch.zeros(num_steps, 8, dtype=torch.float64, device=dev)
         pin = dict(device="cpu", pin_memory=True)
         self._host = (torch.zeros(self.means.shape, **pin), torch.zeros(num_steps, dtype=torch.int32, **pin),
                       torch.zeros(num_steps, dtype=torch.long, **pin))
+        self._host_ranges = (torch.zeros(num_steps, 8, dtype=torch.float64, **pin), torch.zeros(8, dtype=torch.float64, **pin))
 
     @staticmethod
     def logs_terrain(env) -> bool:
@@ -82,13 +106,23 @@ class EpisodeTables:
             torch.sum(env.terrain_levels, dim=0, out=self.terrain_sum[k])
         self.max_command_x[k] = float(env.command_ranges["lin_vel_x"][1])
 
-    def episode_infos(self, env) -> List[Dict]:
+    def episode_infos(self, env, schedule=None) -> List[Dict]:
         """One dict per step that had resets, with _log_episode's keys and values (as Python floats: the tables come
-        to the host in one go, the one host sync of a rollout)."""
+        to the host in one go, the one host sync of a rollout).  schedule = (max_command_x at the start, the steps that
+        ran the device curriculum) when the rollout ran in the device-schedule mode: the device ranges come back in the
+        same batch, command_ranges takes them, and max_command_x is rebuilt from the logged rows."""
         for h, d in zip(self._host, (self.means, self.counts, self.terrain_sum)):
             h.copy_(d, non_blocking=True)
+        if schedule is not None:
+            for h, d in zip(self._host_ranges, (self.ranges_log, env._cmd_ranges_dev)):
+                h.copy_(d, non_blocking=True)
         torch.cuda.current_stream(env.device).synchronize()
         means, counts, tsum = (h.tolist() for h in self._host)
+        if schedule is not None:
+            rows, now = (h.tolist() for h in self._host_ranges)
+            env.set_command_ranges_flat(now)
+            env._cmd_ranges_mirror = tuple(now)
+            self.max_command_x = max_command_x_per_step(schedule[0], schedule[1], rows, len(counts))
         terrain = self.logs_terrain(env)
         names = list(env.episode_sums.keys())
         infos = []
@@ -113,10 +147,19 @@ class RolloutGraph:
 
     Host-side effects of `body` happen only when it runs (eagerly or while capturing); after a replay run() restores
     what T eager steps leave on the host: common_step_counter += T, storage.step, the env's rollout-slot binding and
-    extras.  run() returns the reference's per-step `ep_infos`."""
+    extras.  run() returns the reference's per-step `ep_infos`.
+
+    capture_schedule=True: push and command-curriculum steps are captured too (graphs are cached by the positions of
+    the window's disturbance, push and curriculum steps), so after the warm-up every window replays.  For every window
+    run() executes, eager or replayed, the env is in its device-schedule mode: the kernels read the command ranges
+    from the env's device copy and the curriculum decides on the device (hl_command_curriculum).  run() uploads
+    command_ranges when the host values changed since the last rollout and copies the device ranges back with the
+    episode tables.  A subclass that overrides update_command_curriculum keeps its curriculum windows eager, on the
+    host ranges."""
 
     def __init__(self, env, body: Callable[[int], None], num_steps: int, storage=None,
-                 finish: Optional[Callable[[], None]] = None, max_graphs: int = 8, warmup: int = 1):
+                 finish: Optional[Callable[[], None]] = None, max_graphs: int = 8, warmup: int = 1,
+                 capture_schedule: bool = False):
         if not env._kernel_reset_ok():
             raise ValueError("capture_rollout needs the in-kernel reset (a torch reset hook syncs on the host every step)")
         if getattr(env, "gym", None) is not None:
@@ -125,6 +168,7 @@ class RolloutGraph:
             raise ValueError("num_steps must be positive")
         self.env, self.body, self.num_steps, self.storage, self.finish = env, body, int(num_steps), storage, finish
         self.max_graphs, self.warmup = max(int(max_graphs), 1), int(warmup)
+        self.capture_schedule = bool(capture_schedule)
         self.tables = EpisodeTables(env, self.num_steps)
         self._graphs = OrderedDict()           # key -> (graph, signature, host state after the rollout)
         self._device_counter = None            # what env._step_base holds, when known
@@ -188,38 +232,53 @@ class RolloutGraph:
     def run(self) -> List[Dict]:
         env, T = self.env, self.num_steps
         c = env.common_step_counter
-        key, reason = rollout_window(c, T, **env_schedule(env))
+        device_schedule, schedule = self.capture_schedule, None
+        if device_schedule:
+            key, reason = rollout_window(c, T, **env_schedule(env), in_graph=True)
+            cur = key[2]
+            if cur and not env._device_curriculum_ok():      # the host decides: this window runs eagerly on the host ranges
+                key, reason = None, f"update_command_curriculum is overridden: command-curriculum step at counter {c + 1 + cur[0]}"
+                device_schedule = False
+            else:
+                env._upload_command_ranges()
+                schedule = (env.command_ranges["lin_vel_x"][1], cur if "tracking_lin_vel" in env.episode_sums else ())
+        else:
+            key, reason = rollout_window(c, T, **env_schedule(env))
         if key is not None and self.warmup > 0:
             key, reason = None, "warm-up"
             self.warmup -= 1
-        if key is None:
-            self._steps()
-            env._step_base.fill_(env.common_step_counter)
-            self._device_counter = env.common_step_counter
-            self.stats["eager"] += 1
-            self.last_mode, self.last_reason = "eager", reason
-        else:
-            sig = self._signature()
-            entry = self._graphs.get(key)
-            mode = "replay"
-            if entry is None or entry[1] != sig:
-                self._graphs.pop(key, None)
-                g, after = self._capture()
-                entry = self._graphs[key] = (g, sig, after)
-                while len(self._graphs) > self.max_graphs:
-                    self._graphs.popitem(last=False)
-                mode = "capture+replay"
-            self._graphs.move_to_end(key)
-            g, _, after = entry
-            if self._device_counter != c:
-                env._step_base.fill_(c)
-            g.replay()
-            self._device_counter = c + T
-            self._set_host_state(after)
-            env.common_step_counter = c + T
-            self.stats["replays"] += 1
-            self.last_mode, self.last_reason = mode, None
-        infos = self.tables.episode_infos(env)
+        env._device_schedule = device_schedule
+        try:
+            if key is None:
+                self._steps()
+                env._step_base.fill_(env.common_step_counter)
+                self._device_counter = env.common_step_counter
+                self.stats["eager"] += 1
+                self.last_mode, self.last_reason = "eager", reason
+            else:
+                sig = self._signature()
+                entry = self._graphs.get(key)
+                mode = "replay"
+                if entry is None or entry[1] != sig:
+                    self._graphs.pop(key, None)
+                    g, after = self._capture()
+                    entry = self._graphs[key] = (g, sig, after)
+                    while len(self._graphs) > self.max_graphs:
+                        self._graphs.popitem(last=False)
+                    mode = "capture+replay"
+                self._graphs.move_to_end(key)
+                g, _, after = entry
+                if self._device_counter != c:
+                    env._step_base.fill_(c)
+                g.replay()
+                self._device_counter = c + T
+                self._set_host_state(after)
+                env.common_step_counter = c + T
+                self.stats["replays"] += 1
+                self.last_mode, self.last_reason = mode, None
+        finally:
+            env._device_schedule = False
+        infos = self.tables.episode_infos(env, schedule)
         env.extras["time_outs"] = env.time_out_buf
         if infos:
             env.extras["episode"] = infos[-1]
