@@ -476,6 +476,23 @@ int hl_amp_disc_input(const float* state, const float* next_state, const float* 
                       const float* terminal_states, float* next_state_patched_out /* optional */,
                       float* x_out /* (N,60) */, int64_t n_envs, void* stream);
 
+/* One AMP env-step of HybridPolicyRunner.learn (hybrid_runner.py:184-195 without the discriminator MLP), as one
+ * launch without a host sync or allocation, issued after post_physics_step_device():
+ *   next = get_amp_observations() (LR:406-416); next_with_term = next; next_with_term[reset_ids[:*n_reset]] = terminal_amp
+ *   x_out = cat(normalise(amp_obs), normalise(next_with_term))   (N,60), as hl_amp_disc_input computes it
+ *   ReplayBuffer.insert(amp_obs, next_with_term) (replay_buffer.py:52-68) at the device cursor
+ *   amp_obs = next                                               (in place: (N,30) in/out)
+ * reset_ids ascending with the count on the device; only envs with reset_buf set search them.  norm_stats: (2,30)
+ * float64 [mean; var] of the Normalizer, mean = fp32(mean), std = sqrt(fp32(var + eps)), clamp to +-clip; NULL = no
+ * normaliser.  Row e goes to ring row (cursor[0] + e) mod ring_rows.  cursor: int64 {step, num_samples, ticket}, the
+ * ticket zero between launches; the launch advances num_samples = min(ring_rows, max(step + N, num_samples)) and
+ * step = (step + N) mod ring_rows.  n_envs <= ring_rows. */
+int hl_amp_transition(const float* dof_state, const float* base_lin_vel, const float* base_ang_vel,
+                      const uint8_t* reset_buf, const int64_t* reset_ids, const int32_t* n_reset_dev,
+                      const float* terminal_amp, const double* norm_stats, double eps, float clip, float* amp_obs,
+                      float* x_out, float* ring_states, float* ring_next, int64_t ring_rows, int64_t* cursor,
+                      int64_t n_envs, void* stream);
+
 /* ... and its epilogue -- amp_discriminator.py:64-68,70-72:
  * r = coef * clamp(1 - (d-1)^2/4, min 0); if lerp > 0: r = (1-lerp) r + lerp task_r. */
 int hl_amp_reward(const float* d_logits, const float* task_reward, float coef, float lerp,

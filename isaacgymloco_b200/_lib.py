@@ -96,6 +96,8 @@ EXPORTS = {
     "hl_amp_frame_blend": (c_int32, [_vp, _vp, _vp, _vp, c_int32, _vp, _vp, _vp, _vp, _vp, c_int64, _vp]),
     "hl_amp_gather_pairs": (c_int32, [_vp, _vp, c_int64, _vp, _vp, _vp, c_int64, _vp]),
     "hl_amp_disc_input": (c_int32, [_vp, _vp, _vp, _vp, c_float, _vp, _vp, _vp, _vp, _vp, c_int64, _vp]),
+    "hl_amp_transition": (c_int32, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, c_double, c_float, _vp, _vp, _vp, _vp, c_int64,
+                                    _vp, c_int64, _vp]),
     "hl_amp_reward": (c_int32, [_vp, _vp, c_float, c_float, _vp, c_int64, _vp]),
     "hl_moments_workspace_bytes": (c_int64, [c_int32]),
     "hl_column_moments": (c_int32, [_vp, c_int64, c_int32, _vp, _vp, _vp]),

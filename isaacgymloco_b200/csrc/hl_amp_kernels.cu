@@ -192,6 +192,108 @@ extern "C" int hl_amp_reward(const float* d_logits, const float* task_reward, fl
   return HL_OK;
 }
 
+// ============================================================================= AMP transition of one env-step
+// hybrid_runner.py:184-195 minus the discriminator MLP, for a captured rollout: the next AMP observation (LR:406-416,
+// hl_amp_obs_kernel's columns), the terminal patch with the count read on the device, the normalised discriminator input,
+// the replay-ring insert at the device cursor (replay_buffer.py:52-68) and the carried amp_obs.  CTA = 64 envs: lane t
+// of the first 64 finds env e0+t's terminal row (binary search only where reset_buf is set), then the CTA walks the
+// tile's 64 x 30 columns coalesced.  cursor = {step, num_samples, CTA ticket}: every CTA reads step after
+// griddepcontrol.wait; the last CTA to take a ticket advances the cursor with the reference's arithmetic and re-arms
+// the ticket, so the launch is graph-safe.
+constexpr int TRANS_ENVS = 64, TRANS_THREADS = 256;
+__global__ void __launch_bounds__(TRANS_THREADS) hl_amp_transition_kernel(
+    const float* __restrict__ dof, const float* __restrict__ blv, const float* __restrict__ bav,
+    const unsigned char* __restrict__ reset_buf, const long long* __restrict__ reset_ids, const int* __restrict__ n_reset,
+    const float* __restrict__ terminal, const double* __restrict__ stats, double eps, float clip, float* __restrict__ amp_obs,
+    float* __restrict__ x, float* __restrict__ ring_s, float* __restrict__ ring_n, long long ring_rows,
+    long long* __restrict__ cursor, long long n) {
+  __shared__ float s_mean[HL_AMP_OBS], s_std[HL_AMP_OBS];
+  __shared__ int s_row[TRANS_ENVS];          // terminal row of each env of the tile, -1 = none
+  __shared__ long long s_step, s_nsamp;
+  hl_pdl_enter();
+  const int tid = threadIdx.x;
+  const long long e0 = (long long)blockIdx.x * TRANS_ENVS;
+  const int cnt = (int)(n - e0 < TRANS_ENVS ? n - e0 : TRANS_ENVS);
+  if (tid == 0) {
+    s_step = cursor[0];
+    s_nsamp = cursor[1];
+  }
+  // Normalizer.mean_std_f32(): fp32(mean), sqrt(fp32(var + eps)) with the add in float64
+  if (stats && tid < HL_AMP_OBS) {
+    s_mean[tid] = (float)stats[tid];
+    s_std[tid] = __fsqrt_rn((float)(stats[HL_AMP_OBS + tid] + eps));
+  }
+  if (tid < cnt) {
+    const long long e = e0 + tid;
+    int row = -1;
+    if (reset_buf[e]) {       // reset_buf is set exactly for this step's ids: only these envs search
+      const int m = *n_reset;
+      int lo = 0, hi = m;
+      while (lo < hi) {
+        const int mid = (lo + hi) >> 1;
+        if (reset_ids[mid] < e) lo = mid + 1; else hi = mid;
+      }
+      if (lo < m && reset_ids[lo] == e) row = lo;
+    }
+    s_row[tid] = row;
+  }
+  __syncthreads();
+  const long long step = s_step;
+  for (int i = tid; i < cnt * HL_AMP_OBS; i += TRANS_THREADS) {
+    const int le = i / HL_AMP_OBS, k = i - le * HL_AMP_OBS;
+    const long long e = e0 + le;
+    float nx;
+    if (k < 12) nx = dof[e * 24 + 2 * k];
+    else if (k < 15) nx = blv[e * 3 + (k - 12)];
+    else if (k < 18) nx = bav[e * 3 + (k - 15)];
+    else nx = dof[e * 24 + 2 * (k - 18) + 1];
+    const int row = s_row[le];
+    const float nt = row >= 0 ? terminal[(long long)row * HL_AMP_OBS + k] : nx;
+    const float s = amp_obs[e * HL_AMP_OBS + k];
+    long long r = step + e;                  // step < ring_rows and e < n <= ring_rows
+    if (r >= ring_rows) r -= ring_rows;
+    ring_s[r * HL_AMP_OBS + k] = s;
+    ring_n[r * HL_AMP_OBS + k] = nt;
+    float a = s, b = nt;
+    if (stats) {
+      a = hl_clampf(__fdiv_rn(__fsub_rn(a, s_mean[k]), s_std[k]), -clip, clip);
+      b = hl_clampf(__fdiv_rn(__fsub_rn(b, s_mean[k]), s_std[k]), -clip, clip);
+    }
+    x[e * 60 + k] = a;
+    x[e * 60 + HL_AMP_OBS + k] = b;
+    amp_obs[e * HL_AMP_OBS + k] = nx;        // amp_obs = next_amp_obs.clone(): the un-patched observation
+  }
+  __syncthreads();
+  if (tid == 0) {
+    __threadfence();
+    unsigned long long* ticket = reinterpret_cast<unsigned long long*>(cursor + 2);
+    if (atomicAdd(ticket, 1ull) == (unsigned long long)gridDim.x - 1ull) {   // every other CTA has read the cursor
+      const long long end = step + n, most = end > s_nsamp ? end : s_nsamp;
+      cursor[1] = most < ring_rows ? most : ring_rows;    // min(size, max(step + N, num_samples))
+      cursor[0] = end >= ring_rows ? end - ring_rows : end;   // (step + N) % size
+      *ticket = 0ull;
+    }
+  }
+}
+
+extern "C" int hl_amp_transition(const float* dof_state, const float* base_lin_vel, const float* base_ang_vel,
+                                 const uint8_t* reset_buf, const int64_t* reset_ids, const int32_t* n_reset_dev,
+                                 const float* terminal_amp, const double* norm_stats, double eps, float clip, float* amp_obs,
+                                 float* x_out, float* ring_states, float* ring_next, int64_t ring_rows, int64_t* cursor,
+                                 int64_t n_envs, void* stream) {
+  HL_CHECK_ARG(dof_state && base_lin_vel && base_ang_vel && amp_obs && x_out, "null pointer");
+  HL_CHECK_ARG(reset_buf && reset_ids && n_reset_dev && terminal_amp, "terminal patch needs reset_buf, ids, count and rows");
+  HL_CHECK_ARG(ring_states && ring_next && cursor, "null ring or cursor");
+  HL_CHECK_ARG(ring_rows > 0 && n_envs <= ring_rows, "n_envs must not exceed the ring's rows");
+  if (n_envs <= 0) return HL_OK;
+  const unsigned blocks = (unsigned)((n_envs + TRANS_ENVS - 1) / TRANS_ENVS);
+  hl_launch(hl_amp_transition_kernel, dim3(blocks), dim3(TRANS_THREADS), 0, (cudaStream_t)stream, dof_state, base_lin_vel,
+            base_ang_vel, (const unsigned char*)reset_buf, (const long long*)reset_ids, n_reset_dev, terminal_amp, norm_stats,
+            eps, clip, amp_obs, x_out, ring_states, ring_next, (long long)ring_rows, (long long*)cursor, (long long)n_envs);
+  HL_CHECK_LAUNCH();
+  return HL_OK;
+}
+
 // ============================================================================= a20: batch moments
 // UT:90-94 on device, float64 accumulation (the reference copies the batch to the host and uses
 // numpy): pass 1 = per-block column sums / sums of squares, pass 2 = one block folds them.

@@ -18,6 +18,11 @@ rollout run eagerly:
 torch-RNG hooks inside `body` (_delay_actions, _disturbance_robots, the policy's action sampling) stay torch: PyTorch's
 graph-safe Philox gives them fresh draws on every replay.  A live Isaac Gym sim cannot be captured (gym.simulate is
 a host call); this mode is for standalone, replayed or otherwise capturable physics (physics_step_fn).
+
+amp=AMPRolloutStep (amp_rollout.py): the hybrid runner's AMP step inside `body` (hl_amp_transition, the discriminator
+MLP, hl_amp_reward).  Its replay-ring cursor and normaliser snapshot live on the device; run() refreshes them from the
+host objects at the start of every rollout and, after a replay, moves the replay buffer's host step / num_samples on by
+the inserts the window made.
 """
 from collections import OrderedDict
 from typing import Callable, Dict, List, Optional, Tuple
@@ -149,6 +154,11 @@ class RolloutGraph:
     what T eager steps leave on the host: common_step_counter += T, storage.step, the env's rollout-slot binding and
     extras.  run() returns the reference's per-step `ep_infos`.
 
+    amp (an AMPRolloutStep whose step() `body` calls): its discriminator parameters, ring tensors and buffers join the
+    graph signature (rebinding any of them recaptures; in-place optimizer steps and load_state_dict do not), run()
+    refreshes its normaliser snapshot and device cursor first, and after a replay the replay buffer's host step /
+    num_samples advance by (amp.step() calls in one pass of `body`) x N inserts, as the eager window leaves them.
+
     capture_schedule=True: push and command-curriculum steps are captured too (graphs are cached by the positions of
     the window's disturbance, push and curriculum steps), so after the warm-up every window replays.  For every window
     run() executes, eager or replayed, the env is in its device-schedule mode: the kernels read the command ranges
@@ -159,7 +169,7 @@ class RolloutGraph:
 
     def __init__(self, env, body: Callable[[int], None], num_steps: int, storage=None,
                  finish: Optional[Callable[[], None]] = None, max_graphs: int = 8, warmup: int = 1,
-                 capture_schedule: bool = False):
+                 capture_schedule: bool = False, amp=None):
         if not env._kernel_reset_ok():
             raise ValueError("capture_rollout needs the in-kernel reset (a torch reset hook syncs on the host every step)")
         if getattr(env, "gym", None) is not None:
@@ -169,6 +179,7 @@ class RolloutGraph:
         self.env, self.body, self.num_steps, self.storage, self.finish = env, body, int(num_steps), storage, finish
         self.max_graphs, self.warmup = max(int(max_graphs), 1), int(warmup)
         self.capture_schedule = bool(capture_schedule)
+        self.amp = amp
         self.tables = EpisodeTables(env, self.num_steps)
         self._graphs = OrderedDict()           # key -> (graph, signature, host state after the rollout)
         self._device_counter = None            # what env._step_base holds, when known
@@ -182,12 +193,14 @@ class RolloutGraph:
         env, st = self.env, self.storage
         noise = tuple(None if t is None else t.data_ptr() for t in env._noise.values())
         return (bytes(env._reset_struct()), noise, env.obs_buf.data_ptr(), env.privileged_obs_buf.data_ptr(),
-                st.step if st is not None else None, env.resample_interval)
+                st.step if st is not None else None, env.resample_interval,
+                self.amp.signature() if self.amp is not None else None)
 
     def _host_state(self):
         env, st = self.env, self.storage
         return dict(counter=env.common_step_counter, step=st.step if st is not None else None, obs=env.obs_buf,
-                    priv=env.privileged_obs_buf, extras=dict(env.extras))
+                    priv=env.privileged_obs_buf, extras=dict(env.extras),
+                    amp=self.amp.host_state() if self.amp is not None else None)
 
     def _set_host_state(self, h):
         env, st = self.env, self.storage
@@ -197,6 +210,8 @@ class RolloutGraph:
         env.obs_buf, env.privileged_obs_buf = h["obs"], h["priv"]
         env.extras.clear()
         env.extras.update(h["extras"])
+        if self.amp is not None:
+            self.amp.set_host_state(h["amp"])
 
     def _steps(self):
         env = self.env
@@ -221,6 +236,7 @@ class RolloutGraph:
                 self._steps()
                 env._step_base.add_(self.num_steps)
             after = self._host_state()
+            after["amp_calls"] = after["amp"][3] - before["amp"][3] if self.amp is not None else 0
         finally:
             env._capture_base = None
             self._set_host_state(before)          # the capture executed nothing
@@ -248,6 +264,8 @@ class RolloutGraph:
             key, reason = None, "warm-up"
             self.warmup -= 1
         env._device_schedule = device_schedule
+        if self.amp is not None:
+            self.amp.refresh()
         try:
             if key is None:
                 self._steps()
@@ -270,9 +288,14 @@ class RolloutGraph:
                 g, _, after = entry
                 if self._device_counter != c:
                     env._step_base.fill_(c)
+                amp_before = self.amp.host_state() if self.amp is not None else None
                 g.replay()
                 self._device_counter = c + T
                 self._set_host_state(after)
+                if self.amp is not None:      # the inserts of the replayed window, counted while it was captured
+                    self.amp.set_host_state(amp_before)
+                    self.amp.advance(after["amp_calls"])
+                    self.amp.calls += after["amp_calls"]
                 env.common_step_counter = c + T
                 self.stats["replays"] += 1
                 self.last_mode, self.last_reason = mode, None
