@@ -365,6 +365,20 @@ int hl_command_curriculum(const float* tracking_sums, const int64_t* env_ids, co
 int hl_ring_insert(const float* states, const float* next_states, float* ring_states, float* ring_next,
                    int64_t n_rows, int32_t width, int64_t buffer_rows, int64_t step, void* stream);
 
+/* The runners' episode statistics of one env-step (him_on_policy_runner.py / hybrid_runner.py), as one launch without a
+ * host sync or allocation:
+ *   cur_reward_sum += rewards; cur_episode_length += 1
+ *   new_ids = (dones > 0).nonzero(); rewbuffer.extend(cur_reward_sum[new_ids]); lenbuffer.extend(cur_episode_length[new_ids])
+ *   cur_reward_sum[new_ids] = 0; cur_episode_length[new_ids] = 0
+ * The deques are a device ring of ring_size entries per buffer: entry i of the run goes to slot i mod ring_size, in
+ * ascending env id within a step.  ids: the step's done envs, ascending, count *n_ids_dev on the device (the capacity-N
+ * buffer of post_physics_step_device() will do); only envs with dones set search them.  cursor: int64 {total, ticket},
+ * the ticket zero between launches; total = the entries written so far, advanced by *n_ids_dev.  Of a step with more
+ * done envs than ring_size only the last ring_size are written. */
+int hl_episode_stats(const float* rewards, const uint8_t* dones, const int64_t* ids, const int32_t* n_ids_dev,
+                     float* cur_reward_sum, float* cur_episode_length, float* ring_reward, float* ring_length,
+                     int64_t ring_size, int64_t* cursor, int64_t n_envs, void* stream);
+
 /* reset_idx's episode logging -- LR:346-350: for every reward row k,
  *   means_out[k] = mean_{e in env_ids}( episode_sums[k][e] / clip(episode_length_buf[e], min=1) / dt )
  * (one launch instead of 21 masked-mean chains; the id count stays on the device).  With

@@ -91,6 +91,7 @@ EXPORTS = {
     "hl_sizeof_transition": (c_int32, []),
     "hl_record_transition": (c_int32, [POINTER(HlTransition), c_int64, _vp]),
     "hl_ring_insert": (c_int32, [_vp, _vp, _vp, _vp, c_int64, c_int32, c_int64, c_int64, _vp]),
+    "hl_episode_stats": (c_int32, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, c_int64, _vp, c_int64, _vp]),
     "hl_sizeof_gather_fields": (c_int32, []),
     "hl_minibatch_gather": (c_int32, [POINTER(HlGatherFields), _vp, c_int64, c_int64, _vp]),
     "hl_amp_frame_blend": (c_int32, [_vp, _vp, _vp, _vp, c_int32, _vp, _vp, _vp, _vp, _vp, c_int64, _vp]),

@@ -334,3 +334,68 @@ extern "C" int hl_ring_insert(const float* states, const float* next_states, flo
   HL_CHECK_LAUNCH();
   return HL_OK;
 }
+
+
+// ============================================================================= episode statistics
+// The runner's rewbuffer / lenbuffer bookkeeping of one env-step (see include/himloco_b200.h), one thread per env.  A
+// done env's entry is the j-th of the step (j = rank of its id in the ascending ids, binary search only where dones is
+// set) and goes to ring slot (total + j) mod ring_size; only the last ring_size ranks of a step write, so no two writes
+// of a step share a slot.  cursor = {total, CTA ticket}: every CTA reads total after griddepcontrol.wait; the CTA that
+// takes the last ticket adds the step's count and re-arms the ticket, so the launch is graph-safe.
+constexpr int EPS_THREADS = 256;
+__global__ void __launch_bounds__(EPS_THREADS) hl_episode_stats_kernel(
+    const float* __restrict__ rewards, const unsigned char* __restrict__ dones, const long long* __restrict__ ids,
+    const int* __restrict__ n_ids, float* __restrict__ cur_r, float* __restrict__ cur_l, float* __restrict__ ring_r,
+    float* __restrict__ ring_l, long long ring_size, long long* __restrict__ cursor, long long n) {
+  __shared__ long long s_total;
+  hl_pdl_enter();
+  const int tid = threadIdx.x;
+  if (tid == 0) s_total = cursor[0];
+  __syncthreads();
+  const long long e = (long long)blockIdx.x * EPS_THREADS + tid;
+  if (e < n) {
+    float r = __fadd_rn(cur_r[e], rewards[e]);       // cur_reward_sum += rewards
+    float l = __fadd_rn(cur_l[e], 1.0f);             // cur_episode_length += 1
+    if (dones[e]) {
+      const int m = *n_ids;
+      int lo = 0, hi = m;
+      while (lo < hi) {
+        const int mid = (lo + hi) >> 1;
+        if (ids[mid] < e) lo = mid + 1; else hi = mid;
+      }
+      if (lo < m && ids[lo] == e && (long long)lo >= (long long)m - ring_size) {
+        const long long slot = (s_total + lo) % ring_size;
+        ring_r[slot] = r;
+        ring_l[slot] = l;
+      }
+      r = 0.0f;
+      l = 0.0f;
+    }
+    cur_r[e] = r;
+    cur_l[e] = l;
+  }
+  if (tid == 0) {
+    __threadfence();
+    unsigned long long* ticket = reinterpret_cast<unsigned long long*>(cursor + 1);
+    if (atomicAdd(ticket, 1ull) == (unsigned long long)gridDim.x - 1ull) {   // every other CTA has read total
+      cursor[0] = s_total + *n_ids;
+      *ticket = 0ull;
+    }
+  }
+}
+
+extern "C" int hl_episode_stats(const float* rewards, const uint8_t* dones, const int64_t* ids, const int32_t* n_ids_dev,
+                                float* cur_reward_sum, float* cur_episode_length, float* ring_reward, float* ring_length,
+                                int64_t ring_size, int64_t* cursor, int64_t n_envs, void* stream) {
+  HL_CHECK_ARG(rewards && dones && ids && n_ids_dev, "null input");
+  HL_CHECK_ARG(cur_reward_sum && cur_episode_length, "null running sums");
+  HL_CHECK_ARG(ring_reward && ring_length && cursor, "null ring or cursor");
+  HL_CHECK_ARG(ring_size >= 1, "ring_size must be at least 1");
+  HL_CHECK_ARG(n_envs >= 1, "n_envs must be at least 1");
+  const unsigned blocks = (unsigned)((n_envs + EPS_THREADS - 1) / EPS_THREADS);
+  hl_launch(hl_episode_stats_kernel, dim3(blocks), dim3(EPS_THREADS), 0, (cudaStream_t)stream, rewards,
+            (const unsigned char*)dones, (const long long*)ids, n_ids_dev, cur_reward_sum, cur_episode_length, ring_reward,
+            ring_length, (long long)ring_size, (long long*)cursor, (long long)n_envs);
+  HL_CHECK_LAUNCH();
+  return HL_OK;
+}

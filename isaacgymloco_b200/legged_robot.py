@@ -794,7 +794,7 @@ class FusedLeggedRobot:
                 term_amp)
 
     def capture_rollout(self, body: Callable[[int], None], num_steps: int, storage=None, finish: Optional[Callable[[], None]] = None,
-                        max_graphs: int = 8, warmup: int = 1, capture_schedule: bool = False, amp=None):
+                        max_graphs: int = 8, warmup: int = 1, capture_schedule: bool = False, amp=None, episode_stats=None):
         """A RolloutGraph that runs `body(0) .. body(num_steps - 1)` then `finish()` as one captured CUDA graph whenever
         the rollout window allows it, and eagerly otherwise (rollout_graph.py).  `body(k)` is the runner's per-step
         code (act -> step_device -> storage.record_env_step(..., termination_count=n_reset)); `finish` e.g.
@@ -802,10 +802,12 @@ class FusedLeggedRobot:
         captured graphs; the first `warmup` rollouts run eagerly.  `capture_schedule=True` also replays windows with
         push and command-curriculum steps: inside run() the command ranges live on the device and the curriculum
         decides there (its float64 sum can differ from the host's fp32 mean within a few ulp of the threshold).
-        `amp`: the AMPRolloutStep (amp_rollout.py) whose step() `body` calls, for the hybrid (AMP) runner."""
+        `amp`: the AMPRolloutStep (amp_rollout.py) whose step() `body` calls, for the hybrid (AMP) runner.
+        `episode_stats`: the EpisodeStats (episode_stats.py) whose record() `body` calls; run() fills its rewbuffer /
+        lenbuffer."""
         from .rollout_graph import RolloutGraph
         return RolloutGraph(self, body, num_steps, storage=storage, finish=finish, max_graphs=max_graphs, warmup=warmup,
-                            capture_schedule=capture_schedule, amp=amp)
+                            capture_schedule=capture_schedule, amp=amp, episode_stats=episode_stats)
 
     # ------------------------------------------------------------------ torch-side hooks (RNG / PhysX)
     def _delay_actions(self):

@@ -23,6 +23,10 @@ amp=AMPRolloutStep (amp_rollout.py): the hybrid runner's AMP step inside `body` 
 MLP, hl_amp_reward).  Its replay-ring cursor and normaliser snapshot live on the device; run() refreshes them from the
 host objects at the start of every rollout and, after a replay, moves the replay buffer's host step / num_samples on by
 the inserts the window made.
+
+episode_stats=EpisodeStats (episode_stats.py): the runner's rewbuffer / lenbuffer bookkeeping inside `body`
+(hl_episode_stats, one launch per step).  Its ring and entry count come back in the same copy batch as the episode
+tables, before the one sync, and run() extends the host deques from them.
 """
 from collections import OrderedDict
 from typing import Callable, Dict, List, Optional, Tuple
@@ -159,6 +163,10 @@ class RolloutGraph:
     refreshes its normaliser snapshot and device cursor first, and after a replay the replay buffer's host step /
     num_samples advance by (amp.step() calls in one pass of `body`) x N inserts, as the eager window leaves them.
 
+    episode_stats (an EpisodeStats whose record() `body` calls): its buffer addresses and ring size join the graph
+    signature, and after every window, eager or replayed, run() extends its rewbuffer / lenbuffer by the episodes the
+    window finished, with no sync beyond its one.
+
     capture_schedule=True: push and command-curriculum steps are captured too (graphs are cached by the positions of
     the window's disturbance, push and curriculum steps), so after the warm-up every window replays.  For every window
     run() executes, eager or replayed, the env is in its device-schedule mode: the kernels read the command ranges
@@ -169,17 +177,20 @@ class RolloutGraph:
 
     def __init__(self, env, body: Callable[[int], None], num_steps: int, storage=None,
                  finish: Optional[Callable[[], None]] = None, max_graphs: int = 8, warmup: int = 1,
-                 capture_schedule: bool = False, amp=None):
+                 capture_schedule: bool = False, amp=None, episode_stats=None):
         if not env._kernel_reset_ok():
             raise ValueError("capture_rollout needs the in-kernel reset (a torch reset hook syncs on the host every step)")
         if getattr(env, "gym", None) is not None:
             raise ValueError("capture_rollout needs standalone physics: gym.simulate cannot be captured")
         if num_steps <= 0:
             raise ValueError("num_steps must be positive")
+        if episode_stats is not None and episode_stats.num_envs != env.num_envs:
+            raise ValueError(f"episode_stats keeps {episode_stats.num_envs} envs, the env has {env.num_envs}")
         self.env, self.body, self.num_steps, self.storage, self.finish = env, body, int(num_steps), storage, finish
         self.max_graphs, self.warmup = max(int(max_graphs), 1), int(warmup)
         self.capture_schedule = bool(capture_schedule)
         self.amp = amp
+        self.episode_stats = episode_stats
         self.tables = EpisodeTables(env, self.num_steps)
         self._graphs = OrderedDict()           # key -> (graph, signature, host state after the rollout)
         self._device_counter = None            # what env._step_base holds, when known
@@ -194,7 +205,8 @@ class RolloutGraph:
         noise = tuple(None if t is None else t.data_ptr() for t in env._noise.values())
         return (bytes(env._reset_struct()), noise, env.obs_buf.data_ptr(), env.privileged_obs_buf.data_ptr(),
                 st.step if st is not None else None, env.resample_interval,
-                self.amp.signature() if self.amp is not None else None)
+                self.amp.signature() if self.amp is not None else None,
+                self.episode_stats.signature() if self.episode_stats is not None else None)
 
     def _host_state(self):
         env, st = self.env, self.storage
@@ -301,7 +313,11 @@ class RolloutGraph:
                 self.last_mode, self.last_reason = mode, None
         finally:
             env._device_schedule = False
+        if self.episode_stats is not None:
+            self.episode_stats._enqueue_copies()     # completed by the sync in episode_infos
         infos = self.tables.episode_infos(env, schedule)
+        if self.episode_stats is not None:
+            self.episode_stats._extend()
         env.extras["time_outs"] = env.time_out_buf
         if infos:
             env.extras["episode"] = infos[-1]
