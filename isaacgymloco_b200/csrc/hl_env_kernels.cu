@@ -314,7 +314,7 @@ __device__ __forceinline__ float hl_warp_scan_env(const HlCfg& c, const HlEnvBuf
         aj.a = __shfl_sync(0xffffffffu, axj.a, j);
         aj.c = __shfl_sync(0xffffffffu, axj.c, j);
         const int hraw = hl_scan_point(c, b, posx, posy, c.bx[i], c.by[j], ai, aj, nullptr, nullptr);
-        if (p < P) acc += posz - (float)hraw * c.vertical_scale;
+        if (p < P) acc += posz - __fmul_rn((float)hraw, c.vertical_scale);   // LR:1396: `heights * vertical_scale` rounded before the subtraction (no FMA)
       }
       base_h = warp_sum(acc) / (float)P;
     }

@@ -230,7 +230,7 @@ __device__ float hl_foot_clearance_terrain(const HlCfg& c, const HlEnvBuffers& b
       long long ix = (long long)gx, iy = (long long)gy;
       ix = ix < 0 ? 0 : (ix > c.terrain_rows - 2 ? c.terrain_rows - 2 : ix);
       iy = iy < 0 ? 0 : (iy > c.terrain_cols - 2 ? c.terrain_cols - 2 : iy);
-      fh = sz - (float)hl_sample_min3(c, b, (int)ix, (int)iy) * c.vertical_scale;
+      fh = sz - __fmul_rn((float)hl_sample_min3(c, b, (int)ix, (int)iy), c.vertical_scale);   // LR:1741: `heights * vertical_scale` rounded before the subtraction
     }
     const float lat = sqrtf(hl_sq(v.fvel[f][0]) + hl_sq(v.fvel[f][1]));
     acc += lat * hl_sq(fh - c.foot_height_target_terrain);
