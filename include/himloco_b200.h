@@ -275,6 +275,10 @@ int hl_post_reset_fixup(const HlCfg* cfg, const HlEnvBuffers* bufs, const int64_
  *   36 cmd vx | 37 cmd vy | 38 cmd heading (or yaw rate) | 39 cmd vx of a high-speed env | 40 Kp | 41 Kd |
  *   42 motor strength | 43 random terrain level */
 #define HL_RESET_NU 44
+/* Philox stream map (one stream per draw; the block index and the global env id complete the counter):
+ *   0 observation noise | 1 terminal-observation noise | 2 pre-step command resampling | 3 reset re-draws (columns above)
+ *   4 action delay (hl_delay_actions: word x of block 0) | 5 disturbance (hl_uniform_rows: words 0-2 of block 0) |
+ *   6 push (hl_uniform_rows: words 0-1 of block 0) -- one block per env each. */
 #define HL_RESET_DOFS 1u
 #define HL_RESET_ROOT 2u
 #define HL_RESET_COMMANDS 4u
@@ -357,6 +361,30 @@ int hl_resample_commands(const HlCfg* cfg, const HlEnvBuffers* bufs, const HlRes
 int hl_command_curriculum(const float* tracking_sums, const int64_t* env_ids, const int32_t* n_ids_dev, double threshold,
                           int64_t max_episode_length, double max_backward, double max_forward, double max_lat,
                           double* ranges, double* ranges_log, int64_t n_envs, void* stream);
+
+/* Keyed domain randomisation (opt-in, ResetCfg.keyed_domain_rand): the interval draws of the step from Philox streams
+ * 4-6 keyed by (bufs->philox_seed, the step key of *bufs, cfg->env_id_offset + env), read after griddepcontrol.wait, so
+ * a draw depends on neither the launch mode nor the sharding and a replayed graph draws what eager steps draw.
+ *
+ * step()'s clip and _delay_actions (LR:133-138) in one launch:
+ *   actions_out = torch.clamp(actions_in, -clip_actions, clip_actions)   (NaN passes through; may alias actions_in)
+ *   delay != 0: d = per-env delay in [0, decimation): delay_in[e] (N,) int64 (parity mode) or __umulhi(x, decimation),
+ *               x = word x of Philox block 0, stream 4;
+ *               delayed_out[e,k,:] = last + (actions_out[e,:] - last) * (k >= d ? 1 : 0), last = bufs->last_actions[e,:],
+ *               each op rounded on its own (bit-equal to the torch expression for every input, +-0, +-inf and NaN too)
+ *   delay == 0: delayed_out[e,k,:] = actions_out[e,:] (no draw)
+ * delayed_out: (N, decimation, 12) contiguous; 1 <= decimation <= 16. */
+int hl_delay_actions(const HlCfg* cfg, const HlEnvBuffers* bufs, const float* actions_in, float* actions_out,
+                     float* delayed_out, int32_t decimation, int32_t delay, float clip_actions, const int64_t* delay_in,
+                     int64_t n_envs, void* stream);
+/* torch_rand_float(lo, hi, (N, cols)) written into rows of a strided tensor:
+ *   dst[e*row_stride + c] = fp32(hi - lo) * u + fp32(lo)   (two ops, rounded on their own), c < cols <= 4
+ * u = u_in[e, c] ((N, cols) fp32, parity mode) or hl_u01 of word c of Philox block 0 of `stream_id` (>= 4: streams 0-3
+ * belong to other draws).  _disturbance_robots (LR:838-844): dst = disturbance, row_stride = num_bodies*3, 3 columns,
+ * stream 5.  _push_robots (LR:822-828): dst = root_states + 7, row_stride 13, 2 columns, lo = -max_push_vel_xy, hi =
+ * max_push_vel_xy, stream 6. */
+int hl_uniform_rows(const HlCfg* cfg, const HlEnvBuffers* bufs, float* dst, int64_t row_stride, int32_t cols, double lo,
+                    double hi, const float* u_in, int32_t stream_id, int64_t n_envs, void* stream);
 
 /* ReplayBuffer.insert(states, next_states) -- rsl_rl/rsl_rl/storage/replay_buffer.py:52-68: row r of
  * both (n_rows, width) inputs is written to ring row (step + r) mod buffer_rows; when more than

@@ -7,7 +7,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, os.environ.get("HL_LIB_NAME", "libhimloco_b200.so"))   # HL_LIB_NAME: experiment builds side by side
-SOURCES = ["hl_env_kernels.cu", "hl_rollout_kernels.cu", "hl_amp_kernels.cu"]
+SOURCES = ["hl_env_kernels.cu", "hl_rollout_kernels.cu", "hl_amp_kernels.cu", "hl_domain_rand_kernels.cu"]
 HEADERS = ["hl_common.cuh", "hl_math.cuh", "hl_fused_kernel.inc", "hl_persist_kernel.inc", os.path.join("..", "..", "include", "himloco_b200.h")]
 NVCC_FLAGS = ["-O3", "-std=c++17", "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo",
               "-Xcompiler", "-fPIC", "--shared", "-Xptxas", "-v"]

@@ -202,6 +202,12 @@ class ResetCfg:
     disturbance: bool = True
     disturbance_range: List[float] = field(default_factory=lambda: [-30.0, 30.0])
     delay: bool = True                   # legged_robot.py:134-138
+    # Opt-in: draw the action delay, the disturbances and the pushes from keyed Philox streams 4-6 in the kernel chain
+    # instead of torch's generator -- other numbers than torch draws, but the same ones for every launch mode (eager or
+    # a replayed graph) and every sharding.  Set it on the instance (`cfg.reset.keyed_domain_rand = True`).  It is a
+    # class-level default, not a dataclass field, because it is no setting of the reference: the fields above are the
+    # reference's domain_rand / commands settings, and asdict() of them is what the recorded reference configs hold.
+    keyed_domain_rand = False
 
 
 @dataclass

@@ -4,7 +4,8 @@ names, attribute names, dtypes and in-place side effects, executed by libhimloco
 kernels.
 
 What stays torch / host (out of scope, SURVEY.md §2): PhysX itself and every `gym.*` call (issued here in the
-reference's order when `self.gym` exists), pushes and disturbances (torch RNG written into PhysX-owned tensors),
+reference's order when `self.gym` exists), the action delay, pushes and disturbances (torch RNG written into
+PhysX-owned tensors; with `cfg.reset.keyed_domain_rand` the kernels draw them from keyed Philox streams 4-6 instead),
 the host-side command curriculum, friction re-randomisation.  The reset hooks (`_reset_dofs`, `_reset_root_states`,
 `_resample_commands`, `_update_terrain_curriculum`) run in the kernels by default (Philox, or pre-drawn uniforms in
 parity mode); overriding any of them with torch code (subclass / mix in the reference class, INTEGRATION.md) makes
@@ -184,8 +185,39 @@ class FusedLeggedRobot:
         """Parity mode: the U[0,1) draws `torch.rand_like` would return at LR:394,400 (obs) and
         LR:451,457 (terminal obs).  None => in-kernel Philox."""
         cv = lambda t: None if t is None else t.to(self.device, torch.float32).contiguous()
-        self._noise = dict(obs45=cv(obs45), obs187=cv(obs187), term45=cv(term45), term187=cv(term187))
+        dr = {k: self._noise.get(k) for k in self.DOMAIN_RAND_DRAWS}
+        self._noise = dict(obs45=cv(obs45), obs187=cv(obs187), term45=cv(term45), term187=cv(term187), **dr)
         self._bufs = None
+
+    # parity tensors of the keyed domain randomisation; they live in self._noise beside the noise tensors, so a captured
+    # rollout graph (whose signature covers self._noise) recaptures when they change
+    DOMAIN_RAND_DRAWS = ("delay", "disturbance", "push")
+
+    def set_domain_rand_draws(self, delay=None, disturbance=None, push=None):
+        """Parity mode of cfg.reset.keyed_domain_rand: the draws the kernels take on every step while set, in place of
+        Philox streams 4-6.  delay: (N,) int64 in [0, decimation); disturbance: (N, 3) and push: (N, 2) U[0,1) (any
+        floating dtype, used as float32).  None => in-kernel Philox.  Bad shapes, dtypes or ranges raise ValueError."""
+        n, dec = self.num_envs, self.cfg_hot.decimation
+
+        def check(name, t, shape, lo, hi, integer):
+            if t is None:
+                return None
+            if not isinstance(t, torch.Tensor):
+                raise ValueError(f"{name}: expected a torch.Tensor, got {type(t).__name__}")
+            if integer and t.dtype != torch.int64:
+                raise ValueError(f"{name}: expected int64, got {t.dtype}")
+            if not integer and not t.dtype.is_floating_point:
+                raise ValueError(f"{name}: expected a floating-point tensor, got {t.dtype}")
+            if tuple(t.shape) != shape:
+                raise ValueError(f"{name}: expected shape {shape}, got {tuple(t.shape)}")
+            t = t.to(self.device, torch.int64 if integer else torch.float32).contiguous()
+            if t.numel() and not bool(((t >= lo) & (t < hi)).all()):      # NaN fails too
+                raise ValueError(f"{name}: values must lie in [{lo}, {hi})")
+            return t
+
+        dr = dict(delay=check("delay", delay, (n,), 0, dec, True), disturbance=check("disturbance", disturbance, (n, 3), 0.0, 1.0, False),
+                  push=check("push", push, (n, 2), 0.0, 1.0, False))
+        self._noise = {**self._noise, **dr}
 
     def refresh_buffers(self):
         """Call after rebinding any tensor attribute (pointers are cached in a C struct)."""
@@ -546,18 +578,33 @@ class FusedLeggedRobot:
         return (t._reset_dofs is base._reset_dofs and t._reset_root_states is base._reset_root_states
                 and t._resample_commands is base._resample_commands and t.reset_idx is base.reset_idx)
 
+    def _uniform_rows(self, dst, cols, lo, hi, draws, stream_id):
+        """torch_rand_float(lo, hi, (N, cols)) into the first `cols` columns of the rows of `dst` (row-strided), from
+        Philox stream `stream_id` or the parity tensor self._noise[draws]."""
+        if dst.stride(-1) != 1:
+            raise ValueError("hl_uniform_rows needs unit-stride columns")
+        L.check(L.lib.hl_uniform_rows(ctypes.byref(self._c), ctypes.byref(self._buffers()), L.ptr(dst), dst.stride(0), cols,
+                                      float(lo), float(hi), L.ptr(self._noise.get(draws)), stream_id, self.num_envs, L.stream()))
+
     def _push_robots(self):
-        """LR:822-828 (torch RNG; PhysX-facing)."""
+        """LR:822-828 (torch RNG, or Philox stream 6 with cfg.reset.keyed_domain_rand; PhysX-facing)."""
         mv = self.cfg_hot.reset.max_push_vel_xy
-        self.root_states[:, 7:9] = (2 * mv) * torch.rand(self.num_envs, 2, device=self.device) - mv
+        if self.cfg_hot.reset.keyed_domain_rand:
+            # torch_rand_float(-mv, mv) = (mv - (-mv)) * u + (-mv), bit-equal to the torch form below for every mv
+            self._uniform_rows(self.root_states[:, 7:9], 2, -mv, mv, "push", 6)
+        else:
+            self.root_states[:, 7:9] = (2 * mv) * torch.rand(self.num_envs, 2, device=self.device) - mv
         gym = getattr(self, "gym", None)
         if gym is not None:
             gym.set_actor_root_state_tensor(self.sim, self._uw(self.root_states))
 
     def _disturbance_robots(self):
-        """LR:838-844 (torch RNG; PhysX-facing)."""
+        """LR:838-844 (torch RNG, or Philox stream 5 with cfg.reset.keyed_domain_rand; PhysX-facing)."""
         lo, hi = self.cfg_hot.reset.disturbance_range
-        self.disturbance[:, 0, :] = (hi - lo) * torch.rand(self.num_envs, 3, device=self.device) + lo
+        if self.cfg_hot.reset.keyed_domain_rand:
+            self._uniform_rows(self.disturbance.view(self.num_envs, -1), 3, lo, hi, "disturbance", 5)
+        else:
+            self.disturbance[:, 0, :] = (hi - lo) * torch.rand(self.num_envs, 3, device=self.device) + lo
         gym = getattr(self, "gym", None)
         if gym is not None:
             gym.apply_rigid_body_force_tensors(self.sim, forceTensor=self._uw(self.disturbance), space=getattr(self, "_local_space", "LOCAL_SPACE"))
@@ -751,9 +798,7 @@ class FusedLeggedRobot:
 
     def step(self, actions):
         """LR:122-176.  7-tuple, or the 8-tuple with terminal_amp_states when cfg.using_amp (LR:173-176)."""
-        clip = self.cfg_hot.clip_actions
-        torch.clamp(actions.to(self.device), -clip, clip, out=self.actions)
-        self._delay_actions()
+        self._clip_and_delay(actions)
         gym = getattr(self, "gym", None)
         if gym is not None and hasattr(self, "render"):
             self.render()                                     # LR:131
@@ -780,9 +825,7 @@ class FusedLeggedRobot:
         A live Isaac Gym sim cannot be stepped this way: gym.simulate is a host call that a graph cannot capture."""
         if getattr(self, "gym", None) is not None:
             raise RuntimeError("step_device() needs standalone physics (physics_step_fn): gym.simulate cannot be captured")
-        clip = self.cfg_hot.clip_actions
-        torch.clamp(actions.to(self.device), -clip, clip, out=self.actions)
-        self._delay_actions()
+        self._clip_and_delay(actions)
         for k in range(self.cfg_hot.decimation):
             self._compute_torques_into(self.delayed_actions[:, k], self.torques)
             if self.physics_step_fn is not None:
@@ -810,9 +853,35 @@ class FusedLeggedRobot:
                             capture_schedule=capture_schedule, amp=amp, episode_stats=episode_stats)
 
     # ------------------------------------------------------------------ torch-side hooks (RNG / PhysX)
+    def _clip_and_delay(self, actions):
+        """step()'s action clip and _delay_actions.  With cfg.reset.keyed_domain_rand and the hook not overridden
+        (on the class or the instance) both are one hl_delay_actions launch; otherwise torch.clamp, then the hook."""
+        if self.cfg_hot.reset.keyed_domain_rand and "_delay_actions" not in vars(self) \
+                and type(self)._delay_actions is FusedLeggedRobot._delay_actions:
+            self._launch_delay(actions)
+            return
+        clip = self.cfg_hot.clip_actions
+        torch.clamp(actions.to(self.device), -clip, clip, out=self.actions)
+        self._delay_actions()
+
+    def _launch_delay(self, actions):
+        """hl_delay_actions: self.actions = clamp(actions), delayed_actions from the keyed delay (Philox stream 4, keyed by
+        the step index: common_step_counter before post_physics_step increments it) or the parity delays."""
+        a = actions.to(self.device, torch.float32)
+        if a.shape != self.actions.shape or not a.is_contiguous():
+            a = a.expand_as(self.actions).contiguous()
+        L.check(L.lib.hl_delay_actions(ctypes.byref(self._c), ctypes.byref(self._buffers()), L.ptr(a), L.ptr(self.actions),
+                                       L.ptr(self.delayed_actions), self.cfg_hot.decimation, int(bool(self.cfg_hot.reset.delay)),
+                                       float(self.cfg_hot.clip_actions), L.ptr(self._noise.get("delay")), self.num_envs,
+                                       L.stream()))
+
     def _delay_actions(self):
-        """LR:133-138: per-env random action delay, only when cfg.domain_rand.delay."""
+        """LR:133-138: per-env random action delay, only when cfg.domain_rand.delay (torch RNG, or Philox stream 4 with
+        cfg.reset.keyed_domain_rand)."""
         dec = self.cfg_hot.decimation
+        if self.cfg_hot.reset.keyed_domain_rand:
+            self._launch_delay(self.actions)          # clamping the clipped actions again changes no bit
+            return
         if not self.cfg_hot.reset.delay:
             self.delayed_actions.copy_(self.actions.unsqueeze(1).expand(-1, dec, -1))
             return

@@ -15,8 +15,11 @@ rollout run eagerly:
   sync) is captured as is, and the command ranges and the curriculum decision move to the device (HlReset.cmd_ranges,
   hl_command_curriculum), so windows with either step replay too; graphs are then cached by all three step positions.
 
-torch-RNG hooks inside `body` (_delay_actions, _disturbance_robots, the policy's action sampling) stay torch: PyTorch's
-graph-safe Philox gives them fresh draws on every replay.  A live Isaac Gym sim cannot be captured (gym.simulate is
+The domain-randomisation hooks inside `body` (_delay_actions, _disturbance_robots, _push_robots) draw from torch's
+generator by default: PyTorch's graph-safe Philox gives them fresh draws on every replay, but not the draws the same
+steps take eagerly.  With cfg.reset.keyed_domain_rand they draw from the library's Philox streams 4-6, keyed by the
+step like streams 0-3, so a replay equals the eager steps; the policy's action sampling stays torch in both modes, as
+does any override of the three hooks.  A live Isaac Gym sim cannot be captured (gym.simulate is
 a host call); this mode is for standalone, replayed or otherwise capturable physics (physics_step_fn).
 
 amp=AMPRolloutStep (amp_rollout.py): the hybrid runner's AMP step inside `body` (hl_amp_transition, the discriminator
