@@ -278,7 +278,9 @@ int hl_post_reset_fixup(const HlCfg* cfg, const HlEnvBuffers* bufs, const int64_
 /* Philox stream map (one stream per draw; the block index and the global env id complete the counter):
  *   0 observation noise | 1 terminal-observation noise | 2 pre-step command resampling | 3 reset re-draws (columns above)
  *   4 action delay (hl_delay_actions: word x of block 0) | 5 disturbance (hl_uniform_rows: words 0-2 of block 0) |
- *   6 push (hl_uniform_rows: words 0-1 of block 0) -- one block per env each. */
+ *   6 push (hl_uniform_rows: words 0-1 of block 0) -- one block per env each.
+ *   7 policy action sampling (hl_policy_sample: block b gives the standard normals of actions 4b .. 4b+3,
+ *     ceil(act_dim / 4) blocks per env). */
 #define HL_RESET_DOFS 1u
 #define HL_RESET_ROOT 2u
 #define HL_RESET_COMMANDS 4u
@@ -385,6 +387,25 @@ int hl_delay_actions(const HlCfg* cfg, const HlEnvBuffers* bufs, const float* ac
  * max_push_vel_xy, stream 6. */
 int hl_uniform_rows(const HlCfg* cfg, const HlEnvBuffers* bufs, float* dst, int64_t row_stride, int32_t cols, double lo,
                     double hi, const float* u_in, int32_t stream_id, int64_t n_envs, void* stream);
+/* HIMPPO.act's sampling (him_ppo.py:90; him_actor_critic.py update_distribution / act / get_actions_log_prob /
+ * action_mean / action_std) for Normal(mean, mean*0. + std), one PDL launch, no sync, no allocation.  Per env e and
+ * action j < A = act_dim, each op rounded on its own in torch's order:
+ *   sigma = mean * 0.f + std                  (bit-equal to mean*0. + self.std, NaN / +-inf means and -0 included)
+ *   actions = mean + z * sigma                (rsample()'s loc + eps * scale; also torch.normal(loc, scale))
+ *   mu = mean                                 (skipped when mu_out == mean)
+ *   log_prob[e] = sum_j [ -(d*d) / (2*(s*s)) - logf(s) - fp32(0.9189385332046727) ],  d = actions - mean, s = sigma
+ * The sum over j is sequential (torch's .sum(-1) has its own reduction order; the only intended difference).  sigma is
+ * not validated: a NaN or non-positive std propagates, as with Normal(..., validate_args=False) -- a host-side check
+ * cannot run inside a captured graph.
+ * z = z_in[e, j] ((N, A) standard normals, parity mode) or Philox stream 7 keyed by (bufs->philox_seed, the step key of
+ * *bufs, cfg->env_id_offset + e): block b gives actions 4b .. 4b+3 by Box-Muller on the word pairs (x, y) -> z0, z1 and
+ * (z, w) -> z2, z3: with u(x) = (x >> 8) * 2^-24 (hl_u01), u1 = 1 - u(x) in [2^-24, 1], r = sqrtf(-2 logf(u1)),
+ * (s, c) = sincospif(2 u(y)), z0 = r c, z1 = r s.  Hence |z| <= sqrt(48 ln 2) ~= 5.77.
+ * std: (A,) with std_row_stride 0, or (N, A) with std_row_stride A.  mu_out, sigma_out: (N, A) or NULL.  All (N, A)
+ * tensors are contiguous fp32; log_prob_out is (N,).  1 <= act_dim <= 16. */
+int hl_policy_sample(const HlCfg* cfg, const HlEnvBuffers* bufs, const float* mean, const float* std,
+                     int64_t std_row_stride, const float* z_in, int32_t act_dim, float* actions_out, float* log_prob_out,
+                     float* mu_out, float* sigma_out, int64_t n_envs, void* stream);
 
 /* ReplayBuffer.insert(states, next_states) -- rsl_rl/rsl_rl/storage/replay_buffer.py:52-68: row r of
  * both (n_rows, width) inputs is written to ring row (step + r) mod buffer_rows; when more than

@@ -93,6 +93,8 @@ EXPORTS = {
     "hl_delay_actions": (c_int32, [POINTER(HlCfg), POINTER(HlEnvBuffers), _vp, _vp, _vp, c_int32, c_int32, c_float, _vp, c_int64, _vp]),
     "hl_uniform_rows": (c_int32, [POINTER(HlCfg), POINTER(HlEnvBuffers), _vp, c_int64, c_int32, c_double, c_double, _vp, c_int32,
                                   c_int64, _vp]),
+    "hl_policy_sample": (c_int32, [POINTER(HlCfg), POINTER(HlEnvBuffers), _vp, _vp, c_int64, _vp, c_int32, _vp, _vp, _vp, _vp,
+                                   c_int64, _vp]),
     "hl_ring_insert": (c_int32, [_vp, _vp, _vp, _vp, c_int64, c_int32, c_int64, c_int64, _vp]),
     "hl_episode_stats": (c_int32, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, c_int64, _vp, c_int64, _vp]),
     "hl_sizeof_gather_fields": (c_int32, []),

@@ -1,7 +1,7 @@
 // Keyed domain randomisation (sm_100a): the action delay of step() (LR:133-138, with step()'s clip) and the interval
 // disturbance (LR:838-844) / push (LR:822-828) draws, from Philox streams 4-6 keyed by (seed, step, global env id)
-// like every other in-kernel draw, so they depend on neither the launch mode nor the sharding.  See
-// include/himloco_b200.h for the ABI.
+// like every other in-kernel draw, so they depend on neither the launch mode nor the sharding; and HIMPPO.act's action
+// sampling (him_ppo.py:90) from stream 7.  See include/himloco_b200.h for the ABI.
 #include "hl_common.cuh"
 
 static int check_structs(const HlCfg* c, const HlEnvBuffers* b) {
@@ -118,6 +118,89 @@ extern "C" int hl_uniform_rows(const HlCfg* cfg, const HlEnvBuffers* bufs, float
   hl_launch(hl_uniform_rows_kernel, dim3((unsigned)((n_envs + 255) / 256)), dim3(256), 0, (cudaStream_t)stream, *bufs,
             (long long)cfg->env_id_offset, dst, (long long)row_stride, (int)cols, (float)(hi - lo), (float)lo, u_in,
             (unsigned)stream_id, (long long)n_envs);
+  HL_CHECK_LAUNCH();
+  return HL_OK;
+}
+
+// ============================================================================= policy action sampling
+// CTA = PS_ENVS envs, one thread per env.  Phase 1: the tile's means are staged in shared memory (coalesced).  Phase 2:
+// each thread draws its ceil(A/4) Philox blocks (stream 7), forms sigma, the action and the log-probability terms in
+// column order (the sequential sum), and leaves its actions in shared memory.  Phase 3: actions, mu and sigma are
+// stored as contiguous runs.  Every op is rounded on its own, in the order of torch's Normal (no contraction).
+constexpr int PS_ENVS = 128, PS_MAX_A = 16;
+
+__global__ void __launch_bounds__(PS_ENVS) hl_policy_sample_kernel(HlEnvBuffers b, long long env_off, const float* mean,
+                                                                   const float* __restrict__ std_dev, int std_rows,
+                                                                   const float* __restrict__ z_in, int A, float* act_out,
+                                                                   float* __restrict__ logp_out, float* mu_out,
+                                                                   float* __restrict__ sigma_out, long long n) {
+  __shared__ float s_mean[PS_ENVS * PS_MAX_A], s_act[PS_ENVS * PS_MAX_A];
+  hl_pdl_enter();
+  const int tid = threadIdx.x;
+  const long long e0 = (long long)blockIdx.x * PS_ENVS;
+  const int cnt = (int)((n - e0) < PS_ENVS ? (n - e0) : PS_ENVS);
+  const long long base = e0 * A;
+  for (int i = tid; i < cnt * A; i += PS_ENVS) s_mean[i] = mean[base + i];
+  __syncthreads();
+  if (tid < cnt) {
+    const long long e = e0 + tid;
+    const unsigned long long key = hl_step_key(b);
+    const float* srow = std_rows ? std_dev + e * A : std_dev;
+    float lp = 0.0f;
+    for (int blk = 0; blk * 4 < A; ++blk) {
+      float z[4];
+      if (z_in) {
+        for (int k = 0; k < 4; ++k) z[k] = (blk * 4 + k < A) ? z_in[e * A + blk * 4 + k] : 0.0f;
+      } else {
+        const uint4 q = hl_noise_block(b.philox_seed, key, (unsigned long long)(e + env_off), (unsigned)blk, 7u);
+        // Box-Muller on (x, y) and (z, w): u1 = 1 - u lies in [2^-24, 1], so |z| <= sqrt(-2 ln 2^-24) = sqrt(48 ln 2)
+        const float r0 = sqrtf(__fmul_rn(-2.0f, logf(__fsub_rn(1.0f, hl_u01(q.x)))));
+        const float r1 = sqrtf(__fmul_rn(-2.0f, logf(__fsub_rn(1.0f, hl_u01(q.z)))));
+        float s0, c0, s1, c1;
+        sincospif(__fmul_rn(2.0f, hl_u01(q.y)), &s0, &c0);
+        sincospif(__fmul_rn(2.0f, hl_u01(q.w)), &s1, &c1);
+        z[0] = __fmul_rn(r0, c0);
+        z[1] = __fmul_rn(r0, s0);
+        z[2] = __fmul_rn(r1, c1);
+        z[3] = __fmul_rn(r1, s1);
+      }
+      for (int k = 0; k < 4; ++k) {
+        const int j = blk * 4 + k;
+        if (j >= A) break;
+        const float m = s_mean[tid * A + j];
+        const float sig = __fadd_rn(__fmul_rn(m, 0.0f), srow[j]);          // mean*0. + std
+        const float a = __fadd_rn(m, __fmul_rn(z[k], sig));                  // loc + eps * scale
+        s_act[tid * A + j] = a;
+        // Normal.log_prob: -((value - loc) ** 2) / (2 * var) - log(scale) - log(sqrt(2 pi))
+        const float d = __fsub_rn(a, m);
+        const float q = __fdiv_rn(-__fmul_rn(d, d), __fmul_rn(2.0f, __fmul_rn(sig, sig)));
+        lp = __fadd_rn(lp, __fsub_rn(__fsub_rn(q, logf(sig)), (float)0.9189385332046727));
+      }
+    }
+    logp_out[e] = lp;
+  }
+  __syncthreads();
+  for (int i = tid; i < cnt * A; i += PS_ENVS) {
+    const float m = s_mean[i];
+    act_out[base + i] = s_act[i];
+    if (mu_out) mu_out[base + i] = m;
+    if (sigma_out) sigma_out[base + i] = __fadd_rn(__fmul_rn(m, 0.0f), std_rows ? std_dev[base + i] : std_dev[i % A]);
+  }
+}
+
+extern "C" int hl_policy_sample(const HlCfg* cfg, const HlEnvBuffers* bufs, const float* mean, const float* std_dev,
+                                int64_t std_row_stride, const float* z_in, int32_t act_dim, float* actions_out,
+                                float* log_prob_out, float* mu_out, float* sigma_out, int64_t n_envs, void* stream) {
+  if (int rc = check_structs(cfg, bufs)) return rc;
+  HL_CHECK_ARG(mean && std_dev && actions_out && log_prob_out, "null mean, std, actions_out or log_prob_out");
+  HL_CHECK_ARG(act_dim >= 1 && act_dim <= PS_MAX_A, "act_dim must lie in [1, 16]");
+  HL_CHECK_ARG(std_row_stride == 0 || std_row_stride == act_dim, "std_row_stride must be 0 or act_dim");
+  HL_CHECK_ARG(n_envs >= 0, "negative n_envs");
+  if (n_envs == 0) return HL_OK;
+  hl_launch(hl_policy_sample_kernel, dim3((unsigned)((n_envs + PS_ENVS - 1) / PS_ENVS)), dim3(PS_ENVS), 0,
+            (cudaStream_t)stream, *bufs, (long long)cfg->env_id_offset, mean, std_dev, std_row_stride ? 1 : 0, z_in,
+            (int)act_dim, actions_out, log_prob_out, mu_out == mean ? (float*)nullptr : mu_out, sigma_out,
+            (long long)n_envs);
   HL_CHECK_LAUNCH();
   return HL_OK;
 }

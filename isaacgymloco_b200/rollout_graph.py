@@ -18,9 +18,12 @@ rollout run eagerly:
 The domain-randomisation hooks inside `body` (_delay_actions, _disturbance_robots, _push_robots) draw from torch's
 generator by default: PyTorch's graph-safe Philox gives them fresh draws on every replay, but not the draws the same
 steps take eagerly.  With cfg.reset.keyed_domain_rand they draw from the library's Philox streams 4-6, keyed by the
-step like streams 0-3, so a replay equals the eager steps; the policy's action sampling stays torch in both modes, as
-does any override of the three hooks.  A live Isaac Gym sim cannot be captured (gym.simulate is
-a host call); this mode is for standalone, replayed or otherwise capturable physics (physics_step_fn).
+step like streams 0-3, so a replay equals the eager steps; any override of the three hooks stays torch.  The policy's
+action sampling is torch's unless `body` calls policy_sampling.keyed_act: that draws the actions from stream 7 with the
+same step key (relative to the device counter while a rollout is captured), so with both a replay draws exactly the
+actions, and hence the states, of the same steps run eagerly, with no torch RNG and no host sync left in the rollout.
+A live Isaac Gym sim cannot be captured (gym.simulate is a host call); this mode is for standalone, replayed or
+otherwise capturable physics (physics_step_fn).
 
 amp=AMPRolloutStep (amp_rollout.py): the hybrid runner's AMP step inside `body` (hl_amp_transition, the discriminator
 MLP, hl_amp_reward).  Its replay-ring cursor and normaliser snapshot live on the device; run() refreshes them from the
