@@ -93,13 +93,14 @@ extern "C" int hl_gae_scan(const float* rewards, const float* values, const uint
   return HL_OK;
 }
 
-// advantages = (adv - mean) / (std + 1e-8), std unbiased (torch default) -- :126-127
+// advantages = (adv - mean) / (std + 1e-8), std unbiased (torch default) -- :126-127.  The clamp only removes a
+// negative rounding residue: with one element the variance is 0/0 = NaN, as torch's std() of one element, and stays so.
 __global__ void __launch_bounds__(256) hl_adv_normalize_kernel(float* __restrict__ adv, const double* __restrict__ moments,
                                                                long long n) {
   const double cnt = moments[2];
   const double mean = moments[0] / cnt;
   double var = (moments[1] - moments[0] * mean) / (cnt - 1.0);
-  var = var > 0.0 ? var : 0.0;
+  if (cnt > 1.0) var = var > 0.0 ? var : 0.0;
   const float meanf = (float)mean;
   const float denom = (float)sqrt(var) + 1e-8f;
   const long long i4 = ((long long)blockIdx.x * blockDim.x + threadIdx.x) * 4;

@@ -324,7 +324,17 @@ class FusedLeggedRobot:
         return out
 
     def _compute_torques_into(self, actions, out):
-        """Same, writing into a preallocated (N,12) tensor (no allocation; graph-capturable)."""
+        """Same, writing into a preallocated (N,12) tensor (no allocation; graph-capturable).  `actions` may be
+        row-strided but its columns must be contiguous, and `out` must be a contiguous fp32 (N,12) CUDA tensor: the
+        kernel reads and writes raw pointers, so anything else would be read or written wrong (checked on the
+        strides only: no copy, no sync)."""
+        if actions.dtype != torch.float32 or actions.shape != (self.num_envs, 12) or actions.stride(-1) != 1:
+            raise ValueError(f"actions must be float32 ({self.num_envs}, 12) with unit column stride, got {actions.dtype} "
+                             f"{tuple(actions.shape)} strides {actions.stride()}")
+        if (out.dtype != torch.float32 or out.device != self.dof_state.device or out.shape != (self.num_envs, 12)
+                or not out.is_contiguous()):
+            raise ValueError(f"out must be a contiguous float32 ({self.num_envs}, 12) tensor on {self.dof_state.device}, "
+                             f"got {out.dtype} {tuple(out.shape)} strides {out.stride()} on {out.device}")
         L.check(L.lib.hl_pd_torque(ctypes.byref(self._c), L.ptr(actions), actions.stride(0), L.ptr(self.dof_state),
                                    L.ptr(self.motor_strength), L.ptr(self.Kp_factors), L.ptr(self.Kd_factors),
                                    L.ptr(self.last_dof_vel), L.ptr(out), L.ptr(self.joint_pos_target), self.num_envs,
