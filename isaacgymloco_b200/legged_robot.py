@@ -922,8 +922,9 @@ class FusedLeggedRobot:
         self.last_torques[env_ids] = 0.0
         self.feet_air_time[env_ids] = 0.0
         self.reset_buf[env_ids] = True
-        if type(self)._reset_dofs is FusedLeggedRobot._reset_dofs:   # LR:336-341 (kernel form: same uniform columns)
-            self._reset_part(env_ids, L.RESET_FACTORS)
+        # LR:336-341: reset_idx draws the gain factors itself, after the hooks, whichever of them is overridden
+        # (kernel form: uniform columns 40-42)
+        self._reset_part(env_ids, L.RESET_FACTORS)
         self.extras["episode"] = {}
         if self.episode_sums:   # LR:346-350 as one launch (means of every row over the reset ids, rows zeroed)
             ids, cnt = self._ids_arg(env_ids)

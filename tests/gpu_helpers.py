@@ -27,7 +27,11 @@ def make_env(cfg, state, hf, targets=None, noise=None, no_reset=False, device="c
         def reset_idx(self, ids):
             if self._no_reset:
                 return
+            # the replayed targets carry no gain factors: keep them as they were (reset_idx would re-draw them)
+            factors = [t.clone() for t in (self.Kp_factors, self.Kd_factors, self.motor_strength_factors)]
             super().reset_idx(ids)
+            for t, old in zip((self.Kp_factors, self.Kd_factors, self.motor_strength_factors), factors):
+                t.copy_(old)
 
         def _pre_step_callbacks(self):
             # these tests replay the step without its RNG-driven callbacks (pre-step command resampling,
