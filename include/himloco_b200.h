@@ -280,7 +280,9 @@ int hl_post_reset_fixup(const HlCfg* cfg, const HlEnvBuffers* bufs, const int64_
  *   4 action delay (hl_delay_actions: word x of block 0) | 5 disturbance (hl_uniform_rows: words 0-2 of block 0) |
  *   6 push (hl_uniform_rows: words 0-1 of block 0) -- one block per env each.
  *   7 policy action sampling (hl_policy_sample: block b gives the standard normals of actions 4b .. 4b+3,
- *     ceil(act_dim / 4) blocks per env). */
+ *     ceil(act_dim / 4) blocks per env).
+ *   8 AMP update minibatch rows (hl_amp_update_batch): words x,y the policy ring row, z,w the expert row; one block per
+ *     row, keyed by (seed, the sampler's draw counter, row_offset + row) instead of (seed, step, env). */
 #define HL_RESET_DOFS 1u
 #define HL_RESET_ROOT 2u
 #define HL_RESET_COMMANDS 4u
@@ -560,6 +562,52 @@ int hl_amp_transition(const float* dof_state, const float* base_lin_vel, const f
  * r = coef * clamp(1 - (d-1)^2/4, min 0); if lerp > 0: r = (1-lerp) r + lerp task_r. */
 int hl_amp_reward(const float* d_logits, const float* task_reward, float coef, float lerp,
                   float* reward_out, int64_t n_envs, void* stream);
+
+/* One minibatch of HybridPPO.update's discriminator data path (hybrid_ppo.py:160-281) as one PDL launch, no sync, no
+ * allocation: the rows amp_storage.feed_forward_generator (replay_buffer.py:70-74) and amp_data.feed_forward_generator
+ * (motion_loader.py:315-343, preload branch) draw with host np.random.choice, drawn here from Philox stream 8.  Row r < mb:
+ *   c = draw_counter[0]; n_s = ring_cursor ? ring_cursor[1] : num_samples (0 is read as 1), both after griddepcontrol.wait
+ *   q = Philox block 0 of stream 8 keyed by (seed, offset c, env row_offset + r)
+ *   p = floor(((q.x << 32) | q.y) * n_s / 2^64), e = floor(((q.z << 32) | q.w) * n_preloaded / 2^64)   (bias < n / 2^64)
+ *   or, parity mode, (p, e) = idx_in[r]; idx_out[r] = (p, e) when idx_out is set
+ *   policy_s / policy_sn = ring_states / ring_next[p]; expert_s / expert_sn = columns [7:19] ++ [31:49] of
+ *   preloaded_s / preloaded_s_next[e] (as hl_amp_gather_pairs)
+ *   x_policy = cat(nrm(policy_s), nrm(policy_sn)), x_expert = cat(nrm(expert_s), nrm(expert_sn))   (mb, 60)
+ *   nrm(v) = clamp((v - fp32(mean)) / sqrt(fp32(var + eps)), -clip, clip) (Normalizer.normalize_torch bit for bit);
+ *   norm_mean / norm_var NULL: nrm(v) = v
+ * The CTA that takes the last ticket sets draw_counter[0] = c + 1 and re-arms the ticket (draw_counter = {draws, ticket},
+ * the ticket zero between launches), so launch k draws with key k whether it runs eagerly, captured or replayed.  Every
+ * launch with mb > 0 advances the counter, parity mode included.  Parity rows outside [0, ring_rows) x [0, n_preloaded)
+ * are not written.  All (mb, .) tensors are contiguous fp32, idx_in / idx_out (mb, 2) int64. */
+typedef struct HlAmpUpdateBatch {
+  int32_t struct_bytes;            /* sizeof(HlAmpUpdateBatch): ABI guard */
+  float clip;                      /* Normalizer.clip_obs */
+  const float* ring_states;        /* (ring_rows, 30) ReplayBuffer.states */
+  const float* ring_next;          /* (ring_rows, 30) ReplayBuffer.next_states */
+  int64_t ring_rows;
+  const int64_t* ring_cursor;      /* hl_amp_transition's {step, num_samples, ticket} (only [1] is read) or NULL */
+  int64_t num_samples;             /* the row count when ring_cursor is NULL */
+  const float* preloaded_s;        /* (n_preloaded, 49) AMPLoader.preloaded_s */
+  const float* preloaded_s_next;   /* (n_preloaded, 49) */
+  int64_t n_preloaded;
+  const double* norm_mean;         /* (30,) float64 Normalizer.mean or NULL */
+  const double* norm_var;          /* (30,) float64 Normalizer.var or NULL */
+  double eps;                      /* Normalizer.epsilon */
+  uint64_t seed;
+  int64_t* draw_counter;           /* (2,) {draws, ticket} */
+  int64_t row_offset;              /* global row id of row 0 (rank x mb when envs are sharded) */
+  const int64_t* idx_in;           /* (mb, 2) [policy row, expert row] or NULL => draw */
+  int64_t* idx_out;                /* (mb, 2) or NULL */
+  float* policy_s;
+  float* policy_sn;
+  float* expert_s;
+  float* expert_sn;
+  float* x_policy;
+  float* x_expert;
+  int64_t mb;
+} HlAmpUpdateBatch;
+int hl_sizeof_amp_update_batch(void);
+int hl_amp_update_batch(const HlAmpUpdateBatch* b, void* stream);
 
 /* RunningMeanStd.update moments of one batch -- utils.py:90-94: per-column mean and (biased)
  * variance of x (M,D) in float64; out = [mean(D), var(D)].  Scratch: 2*D*grid doubles provided by

@@ -51,6 +51,15 @@ class HlGatherFields(ctypes.Structure):
                 ("dst", _vp * MAX_GATHER_FIELDS), ("width", c_int32 * MAX_GATHER_FIELDS)]
 
 
+class HlAmpUpdateBatch(ctypes.Structure):
+    """Mirror of `struct HlAmpUpdateBatch` (keep field order identical to the header)."""
+    _fields_ = [("struct_bytes", c_int32), ("clip", c_float), ("ring_states", _vp), ("ring_next", _vp), ("ring_rows", c_int64),
+                ("ring_cursor", _vp), ("num_samples", c_int64), ("preloaded_s", _vp), ("preloaded_s_next", _vp),
+                ("n_preloaded", c_int64), ("norm_mean", _vp), ("norm_var", _vp), ("eps", c_double), ("seed", c_uint64),
+                ("draw_counter", _vp), ("row_offset", c_int64), ("idx_in", _vp), ("idx_out", _vp)] + [(n, _vp) for n in (
+        "policy_s", "policy_sn", "expert_s", "expert_sn", "x_policy", "x_expert")] + [("mb", c_int64)]
+
+
 # stage bits (include/himloco_b200.h)
 ST_COUNTERS, ST_FRAME, ST_CONTACTS, ST_HEADING, ST_HEIGHTS = 0x001, 0x002, 0x004, 0x008, 0x010
 ST_TERMINATION, ST_REWARD, ST_OBS, ST_OBS_NOSHIFT, ST_OBS_CLIP = 0x020, 0x040, 0x080, 0x100, 0x200
@@ -105,6 +114,8 @@ EXPORTS = {
     "hl_amp_transition": (c_int32, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, c_double, c_float, _vp, _vp, _vp, _vp, c_int64,
                                     _vp, c_int64, _vp]),
     "hl_amp_reward": (c_int32, [_vp, _vp, c_float, c_float, _vp, c_int64, _vp]),
+    "hl_sizeof_amp_update_batch": (c_int32, []),
+    "hl_amp_update_batch": (c_int32, [POINTER(HlAmpUpdateBatch), _vp]),
     "hl_moments_workspace_bytes": (c_int64, [c_int32]),
     "hl_column_moments": (c_int32, [_vp, c_int64, c_int32, _vp, _vp, _vp]),
 }
@@ -132,6 +143,9 @@ def _load():
     if lib.hl_sizeof_transition() != ctypes.sizeof(HlTransition):
         raise ImportError(f"HlTransition layout mismatch: python {ctypes.sizeof(HlTransition)} vs "
                           f"library {lib.hl_sizeof_transition()}")
+    if lib.hl_sizeof_amp_update_batch() != ctypes.sizeof(HlAmpUpdateBatch):
+        raise ImportError(f"HlAmpUpdateBatch layout mismatch: python {ctypes.sizeof(HlAmpUpdateBatch)} vs "
+                          f"library {lib.hl_sizeof_amp_update_batch()}")
     return lib
 
 

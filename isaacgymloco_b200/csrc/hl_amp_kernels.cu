@@ -294,6 +294,110 @@ extern "C" int hl_amp_transition(const float* dof_state, const float* base_lin_v
   return HL_OK;
 }
 
+// ============================================================================= AMP update minibatch
+// HybridPPO.update's two discriminator batches (hybrid_ppo.py:160-281): amp_storage.feed_forward_generator's ring rows
+// (replay_buffer.py:70-74), amp_data.feed_forward_generator's preload pairs (ML:315-343) and the normalised 60-wide
+// inputs, for rows drawn from Philox stream 8 instead of host np.random.choice.  CTA = 64 rows: lane t of the first 64
+// draws (or reads) row r0+t's two indices into shared memory, then the CTA walks the tile's 64 x 30 columns coalesced
+// and writes the four raw states and both normalised inputs.  draw_counter = {draws, CTA ticket}: every CTA reads the
+// key after griddepcontrol.wait; the last CTA to take a ticket advances it and re-arms the ticket (graph-safe).
+constexpr int UPD_ROWS = 64, UPD_THREADS = 256;
+__global__ void __launch_bounds__(UPD_THREADS) hl_amp_update_batch_kernel(HlAmpUpdateBatch a) {
+  __shared__ float s_mean[HL_AMP_OBS], s_std[HL_AMP_OBS];
+  __shared__ long long s_p[UPD_ROWS], s_x[UPD_ROWS];   // policy ring row, expert preload row; -1 = out of range
+  __shared__ long long s_key, s_ns;
+  hl_pdl_enter();
+  const int tid = threadIdx.x;
+  const long long r0 = (long long)blockIdx.x * UPD_ROWS;
+  const int cnt = (int)(a.mb - r0 < UPD_ROWS ? a.mb - r0 : UPD_ROWS);
+  const bool norm = a.norm_mean != nullptr;
+  if (tid == 0) {
+    s_key = a.draw_counter[0];
+    const long long ns = a.ring_cursor ? a.ring_cursor[1] : a.num_samples;
+    s_ns = ns < 1 ? 1 : ns;
+  }
+  // Normalizer.mean_std_f32(): fp32(mean), sqrt(fp32(var + eps)) with the add in float64
+  if (norm && tid < HL_AMP_OBS) {
+    s_mean[tid] = (float)a.norm_mean[tid];
+    s_std[tid] = __fsqrt_rn((float)(a.norm_var[tid] + a.eps));
+  }
+  __syncthreads();
+  if (tid < cnt) {
+    const long long r = r0 + tid;
+    long long p, x;
+    if (a.idx_in) {
+      p = a.idx_in[2 * r];
+      x = a.idx_in[2 * r + 1];
+    } else {
+      // floor(u n / 2^64) of a 64-bit word: bias below n / 2^64
+      const uint4 q = hl_noise_block(a.seed, (uint64_t)s_key, (uint64_t)(a.row_offset + r), 0u, 8u);
+      p = (long long)__umul64hi(((unsigned long long)q.x << 32) | q.y, (unsigned long long)s_ns);
+      x = (long long)__umul64hi(((unsigned long long)q.z << 32) | q.w, (unsigned long long)a.n_preloaded);
+    }
+    if (a.idx_out) {
+      a.idx_out[2 * r] = p;
+      a.idx_out[2 * r + 1] = x;
+    }
+    const bool ok = p >= 0 && p < a.ring_rows && x >= 0 && x < a.n_preloaded;   // parity indices out of range: skipped
+    s_p[tid] = ok ? p : -1;
+    s_x[tid] = ok ? x : -1;
+  }
+  __syncthreads();
+  const float clip = a.clip;
+  for (int i = tid; i < cnt * HL_AMP_OBS; i += UPD_THREADS) {
+    const int lr = i / HL_AMP_OBS, k = i - lr * HL_AMP_OBS;
+    const long long p = s_p[lr], x = s_x[lr];
+    if (p < 0) continue;
+    const long long r = r0 + lr;
+    const int src = k < 12 ? 7 + k : 31 + (k - 12);          // expert columns [7:19] ++ [31:49]
+    const float ps = __ldg(a.ring_states + p * HL_AMP_OBS + k), pn = __ldg(a.ring_next + p * HL_AMP_OBS + k);
+    const float es = __ldg(a.preloaded_s + x * HL_AMP_FRAME + src), en = __ldg(a.preloaded_s_next + x * HL_AMP_FRAME + src);
+    a.policy_s[r * HL_AMP_OBS + k] = ps;
+    a.policy_sn[r * HL_AMP_OBS + k] = pn;
+    a.expert_s[r * HL_AMP_OBS + k] = es;
+    a.expert_sn[r * HL_AMP_OBS + k] = en;
+    float v0 = ps, v1 = pn, v2 = es, v3 = en;
+    if (norm) {
+      const float m = s_mean[k], s = s_std[k];
+      v0 = hl_clampf(__fdiv_rn(__fsub_rn(v0, m), s), -clip, clip);
+      v1 = hl_clampf(__fdiv_rn(__fsub_rn(v1, m), s), -clip, clip);
+      v2 = hl_clampf(__fdiv_rn(__fsub_rn(v2, m), s), -clip, clip);
+      v3 = hl_clampf(__fdiv_rn(__fsub_rn(v3, m), s), -clip, clip);
+    }
+    a.x_policy[r * 60 + k] = v0;
+    a.x_policy[r * 60 + HL_AMP_OBS + k] = v1;
+    a.x_expert[r * 60 + k] = v2;
+    a.x_expert[r * 60 + HL_AMP_OBS + k] = v3;
+  }
+  __syncthreads();
+  if (tid == 0) {
+    __threadfence();
+    unsigned long long* ticket = reinterpret_cast<unsigned long long*>(a.draw_counter + 1);
+    if (atomicAdd(ticket, 1ull) == (unsigned long long)gridDim.x - 1ull) {   // every other CTA has read the key
+      a.draw_counter[0] = s_key + 1;
+      *ticket = 0ull;
+    }
+  }
+}
+
+extern "C" int hl_sizeof_amp_update_batch(void) { return (int)sizeof(HlAmpUpdateBatch); }
+
+extern "C" int hl_amp_update_batch(const HlAmpUpdateBatch* b, void* stream) {
+  HL_CHECK_ARG(b, "null argument struct");
+  HL_CHECK_ARG(b->struct_bytes == (int32_t)sizeof(HlAmpUpdateBatch), "HlAmpUpdateBatch layout mismatch");
+  HL_CHECK_ARG(b->ring_states && b->ring_next && b->ring_rows > 0, "null or empty replay ring");
+  HL_CHECK_ARG(b->preloaded_s && b->preloaded_s_next && b->n_preloaded > 0, "null or empty preload tables");
+  HL_CHECK_ARG((b->norm_mean == nullptr) == (b->norm_var == nullptr), "norm_mean and norm_var go together");
+  HL_CHECK_ARG(b->draw_counter, "null draw counter");
+  HL_CHECK_ARG(b->policy_s && b->policy_sn && b->expert_s && b->expert_sn && b->x_policy && b->x_expert, "null output");
+  HL_CHECK_ARG(b->row_offset >= 0, "negative row_offset");
+  if (b->mb <= 0) return HL_OK;
+  const unsigned blocks = (unsigned)((b->mb + UPD_ROWS - 1) / UPD_ROWS);
+  hl_launch(hl_amp_update_batch_kernel, dim3(blocks), dim3(UPD_THREADS), 0, (cudaStream_t)stream, *b);
+  HL_CHECK_LAUNCH();
+  return HL_OK;
+}
+
 // ============================================================================= a20: batch moments
 // UT:90-94 on device, float64 accumulation (the reference copies the batch to the host and uses
 // numpy): pass 1 = per-block column sums / sums of squares, pass 2 = one block folds them.
