@@ -609,6 +609,34 @@ typedef struct HlAmpUpdateBatch {
 int hl_sizeof_amp_update_batch(void);
 int hl_amp_update_batch(const HlAmpUpdateBatch* b, void* stream);
 
+/* Non-finite detection for a rollout step, as one PDL launch without a host sync or allocation.  The kernels clamp
+ * with fminf(fmaxf(x, lo), hi), which turns a NaN into the lower bound (torch.clip keeps it), so a diverged policy or
+ * physics state shows up as finite observations, torques and rewards; this scans the sources before those clamps.
+ * Field k has n_rows rows of width[k] fp32 values, row e column c at src[e*row_stride + c].  An element is flagged
+ *   HL_FINITE:           NaN (any payload or sign), +inf, -inf
+ *   HL_FINITE_POSITIVE:  the same, and every x with !(x > 0) (+0, -0, negatives, negative subnormals): a valid scale
+ * record_out: (n_fields, 3) int64, row k = {count of flagged elements, smallest flagged linear index e*width + c or -1,
+ * the fp32 bits of that element sign-extended from int32 (0 when none)}.
+ * workspace: HL_FINITE_WORKSPACE_WORDS uint64 = {counts[16], first indices[16], CTA ticket}, armed as {0.., ~0.., 0}
+ * before the first launch; the CTA that takes the last ticket writes record_out and re-arms it, so consecutive launches
+ * (and replays of a captured one) are independent without a memset. */
+#define HL_MAX_FINITE_FIELDS 16
+#define HL_FINITE_WORKSPACE_WORDS (2 * HL_MAX_FINITE_FIELDS + 1)
+enum { HL_FINITE = 0, HL_FINITE_POSITIVE = 1 };
+typedef struct HlFiniteField {
+  const float* src;
+  int64_t row_stride;              /* elements between rows, >= width */
+  int32_t width;                   /* >= 1 */
+  int32_t kind;                    /* HL_FINITE or HL_FINITE_POSITIVE */
+} HlFiniteField;
+typedef struct HlFiniteFields {
+  int32_t struct_bytes;            /* sizeof(HlFiniteFields): ABI guard */
+  int32_t n_fields;                /* 1 .. HL_MAX_FINITE_FIELDS */
+  HlFiniteField field[HL_MAX_FINITE_FIELDS];
+} HlFiniteFields;
+int hl_sizeof_finite_fields(void);
+int hl_finite_scan(const HlFiniteFields* f, int64_t n_rows, int64_t* record_out, uint64_t* workspace, void* stream);
+
 /* RunningMeanStd.update moments of one batch -- utils.py:90-94: per-column mean and (biased)
  * variance of x (M,D) in float64; out = [mean(D), var(D)].  Scratch: 2*D*grid doubles provided by
  * the caller via hl_moments_workspace_bytes. */

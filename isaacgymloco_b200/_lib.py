@@ -60,6 +60,21 @@ class HlAmpUpdateBatch(ctypes.Structure):
         "policy_s", "policy_sn", "expert_s", "expert_sn", "x_policy", "x_expert")] + [("mb", c_int64)]
 
 
+MAX_FINITE_FIELDS = 16
+FINITE_WORKSPACE_WORDS = 2 * MAX_FINITE_FIELDS + 1
+FINITE, FINITE_POSITIVE = 0, 1          # HlFiniteField.kind
+
+
+class HlFiniteField(ctypes.Structure):
+    """Mirror of `struct HlFiniteField`."""
+    _fields_ = [("src", _vp), ("row_stride", c_int64), ("width", c_int32), ("kind", c_int32)]
+
+
+class HlFiniteFields(ctypes.Structure):
+    """Mirror of `struct HlFiniteFields`."""
+    _fields_ = [("struct_bytes", c_int32), ("n_fields", c_int32), ("field", HlFiniteField * MAX_FINITE_FIELDS)]
+
+
 # stage bits (include/himloco_b200.h)
 ST_COUNTERS, ST_FRAME, ST_CONTACTS, ST_HEADING, ST_HEIGHTS = 0x001, 0x002, 0x004, 0x008, 0x010
 ST_TERMINATION, ST_REWARD, ST_OBS, ST_OBS_NOSHIFT, ST_OBS_CLIP = 0x020, 0x040, 0x080, 0x100, 0x200
@@ -116,6 +131,8 @@ EXPORTS = {
     "hl_amp_reward": (c_int32, [_vp, _vp, c_float, c_float, _vp, c_int64, _vp]),
     "hl_sizeof_amp_update_batch": (c_int32, []),
     "hl_amp_update_batch": (c_int32, [POINTER(HlAmpUpdateBatch), _vp]),
+    "hl_sizeof_finite_fields": (c_int32, []),
+    "hl_finite_scan": (c_int32, [POINTER(HlFiniteFields), c_int64, _vp, _vp, _vp]),
     "hl_moments_workspace_bytes": (c_int64, [c_int32]),
     "hl_column_moments": (c_int32, [_vp, c_int64, c_int32, _vp, _vp, _vp]),
 }
@@ -146,6 +163,9 @@ def _load():
     if lib.hl_sizeof_amp_update_batch() != ctypes.sizeof(HlAmpUpdateBatch):
         raise ImportError(f"HlAmpUpdateBatch layout mismatch: python {ctypes.sizeof(HlAmpUpdateBatch)} vs "
                           f"library {lib.hl_sizeof_amp_update_batch()}")
+    if lib.hl_sizeof_finite_fields() != ctypes.sizeof(HlFiniteFields):
+        raise ImportError(f"HlFiniteFields layout mismatch: python {ctypes.sizeof(HlFiniteFields)} vs "
+                          f"library {lib.hl_sizeof_finite_fields()}")
     return lib
 
 

@@ -400,3 +400,174 @@ extern "C" int hl_episode_stats(const float* rewards, const uint8_t* dones, cons
   HL_CHECK_LAUNCH();
   return HL_OK;
 }
+
+
+// ============================================================================= non-finite scan
+// Every field is cut into chunks of FS_CHUNK elements, one CTA each; CTAs of field k are [cta_end[k-1], cta_end[k]).  A
+// contiguous field (row_stride == width) is read as 16-B vectors from its first 16-B boundary on, the up to 3 elements
+// before it by the field's first CTA and the up to 3 after the last vector by its last CTA; a strided one element-wise
+// (consecutive threads, consecutive columns).  A CTA reduces its flags in registers and shared memory and, only when it
+// found something, adds its count and folds its smallest index into the workspace (one atomic each per field); the CTA
+// that takes the last ticket reads and re-arms the accumulators, writes the record rows and re-arms the ticket.
+constexpr int FS_THREADS = 256, FS_UNROLL = 8, FS_CHUNK = FS_THREADS * FS_UNROLL * 4;
+
+struct FsArgs {
+  HlFiniteFields f;
+  int32_t cta_end[HL_MAX_FINITE_FIELDS];
+  long long n_rows;
+  long long* record;
+  unsigned long long* ws;
+};
+
+// elements before the first 16-B boundary of a contiguous field (capped by its size)
+__host__ __device__ __forceinline__ long long fs_head(const float* p, long long total) {
+  const long long h = (long long)(((16u - ((unsigned)(uintptr_t)p & 15u)) & 15u) >> 2);
+  return h < total ? h : total;
+}
+__host__ __device__ __forceinline__ long long fs_ctas(const HlFiniteField& d, long long n_rows) {
+  const long long total = n_rows * d.width;
+  if (d.row_stride != d.width) return (total + FS_CHUNK - 1) / FS_CHUNK;
+  const long long body4 = (total - fs_head(d.src, total)) >> 2;
+  const long long c = (body4 + FS_CHUNK / 4 - 1) / (FS_CHUNK / 4);
+  return c > 0 ? c : 1;
+}
+
+__device__ __forceinline__ bool fs_bad(float x, int kind) {
+  const unsigned b = __float_as_uint(x);
+  return (b & 0x7f800000u) == 0x7f800000u || (kind == HL_FINITE_POSITIVE && (int)b <= 0);
+}
+
+__global__ void __launch_bounds__(FS_THREADS) hl_finite_scan_kernel(const FsArgs a) {
+  __shared__ unsigned s_cnt[FS_THREADS / 32];
+  __shared__ unsigned long long s_first[FS_THREADS / 32];
+  __shared__ int s_last;
+  hl_pdl_enter();
+  const int tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
+  int k = 0;
+  while ((int)blockIdx.x >= a.cta_end[k]) ++k;
+  const int j = (int)blockIdx.x - (k ? a.cta_end[k - 1] : 0);
+  const HlFiniteField d = a.f.field[k];
+  const long long total = a.n_rows * d.width;
+  unsigned cnt = 0;
+  unsigned long long first = ~0ull;
+  auto note = [&](float x, long long i) {
+    if (fs_bad(x, d.kind)) {
+      ++cnt;
+      first = (unsigned long long)i < first ? (unsigned long long)i : first;
+    }
+  };
+  if (d.row_stride == d.width) {
+    const long long h = fs_head(d.src, total), body4 = (total - h) >> 2;
+    const float4* v = reinterpret_cast<const float4*>(d.src + h);
+    const long long q0 = (long long)j * (FS_CHUNK / 4), q1 = q0 + FS_CHUNK / 4 < body4 ? q0 + FS_CHUNK / 4 : body4;
+    float4 x[FS_UNROLL];
+#pragma unroll
+    for (int u = 0; u < FS_UNROLL; ++u) {
+      const long long q = q0 + u * FS_THREADS + tid;
+      x[u] = q < q1 ? __ldg(v + q) : make_float4(0.f, 0.f, 0.f, 0.f);
+    }
+#pragma unroll
+    for (int u = 0; u < FS_UNROLL; ++u) {
+      const long long q = q0 + u * FS_THREADS + tid, i = h + 4 * q;
+      if (q < q1) {
+        note(x[u].x, i);
+        note(x[u].y, i + 1);
+        note(x[u].z, i + 2);
+        note(x[u].w, i + 3);
+      }
+    }
+    if (j == 0 && tid < h) note(__ldg(d.src + tid), tid);
+    const long long t0 = h + 4 * body4;
+    if (j == a.cta_end[k] - (k ? a.cta_end[k - 1] : 0) - 1 && t0 + tid < total) note(__ldg(d.src + t0 + tid), t0 + tid);
+  } else {
+    const long long i0 = (long long)j * FS_CHUNK, i1 = i0 + FS_CHUNK < total ? i0 + FS_CHUNK : total;
+    for (long long b = i0; b < i1; b += FS_THREADS * FS_UNROLL) {
+      float x[FS_UNROLL];
+#pragma unroll
+      for (int u = 0; u < FS_UNROLL; ++u) {
+        const long long i = b + u * FS_THREADS + tid;
+        if (i < i1) {
+          const long long e = i / d.width;
+          x[u] = __ldg(d.src + e * d.row_stride + (i - e * d.width));
+        } else {
+          x[u] = 0.f;
+        }
+      }
+#pragma unroll
+      for (int u = 0; u < FS_UNROLL; ++u)
+        if (b + u * FS_THREADS + tid < i1) note(x[u], b + u * FS_THREADS + tid);
+    }
+  }
+  if (__syncthreads_or(cnt != 0)) {            // a clean chunk skips the reduction and the accumulator atomics
+    unsigned c = __reduce_add_sync(0xffffffffu, cnt);
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+      const unsigned long long y = __shfl_xor_sync(0xffffffffu, first, o);
+      first = y < first ? y : first;
+    }
+    if (lane == 0) { s_cnt[wid] = c; s_first[wid] = first; }
+    __syncthreads();
+    if (tid == 0) {
+      c = 0;
+      for (int w = 0; w < FS_THREADS / 32; ++w) {
+        c += s_cnt[w];
+        first = s_first[w] < first ? s_first[w] : first;
+      }
+      atomicAdd(a.ws + k, (unsigned long long)c);
+      atomicMin(a.ws + HL_MAX_FINITE_FIELDS + k, first);
+    }
+  }
+  if (tid == 0) {
+    __threadfence();
+    s_last = atomicAdd(a.ws + 2 * HL_MAX_FINITE_FIELDS, 1ull) == (unsigned long long)gridDim.x - 1ull;
+  }
+  __syncthreads();
+  if (!s_last) return;
+  __threadfence();
+  for (int f = tid; f < a.f.n_fields; f += FS_THREADS) {       // every other CTA has added its flags
+    const unsigned long long n = atomicExch(a.ws + f, 0ull);
+    const unsigned long long i = atomicExch(a.ws + HL_MAX_FINITE_FIELDS + f, ~0ull);
+    const HlFiniteField g = a.f.field[f];
+    long long bits = 0;
+    if (n) {
+      const long long e = (long long)(i / (unsigned long long)g.width);
+      bits = (long long)__float_as_int(g.src[e * g.row_stride + ((long long)i - e * g.width)]);
+    }
+    a.record[3 * f + 0] = (long long)n;
+    a.record[3 * f + 1] = n ? (long long)i : -1ll;
+    a.record[3 * f + 2] = bits;
+  }
+  if (tid == 0) a.ws[2 * HL_MAX_FINITE_FIELDS] = 0ull;
+}
+
+extern "C" int hl_sizeof_finite_fields(void) { return (int)sizeof(HlFiniteFields); }
+extern "C" int hl_finite_scan(const HlFiniteFields* f, int64_t n_rows, int64_t* record_out, uint64_t* workspace,
+                              void* stream) {
+  HL_CHECK_ARG(f && f->struct_bytes == (int)sizeof(HlFiniteFields), "HlFiniteFields size mismatch (ABI)");
+  HL_CHECK_ARG(record_out && workspace, "null record or workspace");
+  HL_CHECK_ARG(f->n_fields >= 1 && f->n_fields <= HL_MAX_FINITE_FIELDS, "n_fields must lie in [1, 16]");
+  HL_CHECK_ARG(n_rows >= 1, "n_rows must be at least 1");
+  FsArgs a;
+  a.f = *f;
+  a.n_rows = (long long)n_rows;
+  a.record = (long long*)record_out;
+  a.ws = (unsigned long long*)workspace;
+  long long ctas = 0;
+  for (int k = 0; k < HL_MAX_FINITE_FIELDS; ++k) {
+    if (k < f->n_fields) {
+      const HlFiniteField& d = f->field[k];
+      HL_CHECK_ARG(d.src, "null field");
+      HL_CHECK_ARG(((uintptr_t)d.src & 3) == 0, "field not 4-byte aligned");
+      HL_CHECK_ARG(d.width >= 1, "width must be at least 1");
+      HL_CHECK_ARG(d.row_stride >= d.width, "row_stride below width");
+      HL_CHECK_ARG(d.kind == HL_FINITE || d.kind == HL_FINITE_POSITIVE, "unknown kind");
+      HL_CHECK_ARG(n_rows <= INT64_MAX / d.row_stride, "field too large");
+      ctas += fs_ctas(d, n_rows);
+      HL_CHECK_ARG(ctas <= 0x7fffffffLL, "too many elements for one launch");
+    }
+    a.cta_end[k] = (int32_t)ctas;
+  }
+  hl_launch(hl_finite_scan_kernel, dim3((unsigned)ctas), dim3(FS_THREADS), 0, (cudaStream_t)stream, a);
+  HL_CHECK_LAUNCH();
+  return HL_OK;
+}

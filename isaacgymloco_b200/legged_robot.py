@@ -847,7 +847,8 @@ class FusedLeggedRobot:
                 term_amp)
 
     def capture_rollout(self, body: Callable[[int], None], num_steps: int, storage=None, finish: Optional[Callable[[], None]] = None,
-                        max_graphs: int = 8, warmup: int = 1, capture_schedule: bool = False, amp=None, episode_stats=None):
+                        max_graphs: int = 8, warmup: int = 1, capture_schedule: bool = False, amp=None, episode_stats=None,
+                        finite_guard=None):
         """A RolloutGraph that runs `body(0) .. body(num_steps - 1)` then `finish()` as one captured CUDA graph whenever
         the rollout window allows it, and eagerly otherwise (rollout_graph.py).  `body(k)` is the runner's per-step
         code (act -> step_device -> storage.record_env_step(..., termination_count=n_reset)); `finish` e.g.
@@ -857,10 +858,12 @@ class FusedLeggedRobot:
         decides there (its float64 sum can differ from the host's fp32 mean within a few ulp of the threshold).
         `amp`: the AMPRolloutStep (amp_rollout.py) whose step() `body` calls, for the hybrid (AMP) runner.
         `episode_stats`: the EpisodeStats (episode_stats.py) whose record() `body` calls; run() fills its rewbuffer /
-        lenbuffer."""
+        lenbuffer.  `finite_guard`: the FiniteGuard (finite_guard.py) whose record(k) `body` calls; run() raises
+        NonFiniteError after a window that produced NaN / Inf."""
         from .rollout_graph import RolloutGraph
         return RolloutGraph(self, body, num_steps, storage=storage, finish=finish, max_graphs=max_graphs, warmup=warmup,
-                            capture_schedule=capture_schedule, amp=amp, episode_stats=episode_stats)
+                            capture_schedule=capture_schedule, amp=amp, episode_stats=episode_stats,
+                            finite_guard=finite_guard)
 
     # ------------------------------------------------------------------ torch-side hooks (RNG / PhysX)
     def _clip_and_delay(self, actions):

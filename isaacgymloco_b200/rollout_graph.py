@@ -33,6 +33,10 @@ the inserts the window made.
 episode_stats=EpisodeStats (episode_stats.py): the runner's rewbuffer / lenbuffer bookkeeping inside `body`
 (hl_episode_stats, one launch per step).  Its ring and entry count come back in the same copy batch as the episode
 tables, before the one sync, and run() extends the host deques from them.
+
+finite_guard=FiniteGuard (finite_guard.py): one hl_finite_scan launch per step inside `body`.  run() zeroes its table
+before the window, copies it back in the same batch, and raises NonFiniteError once the window's host bookkeeping is
+done, so the env is consistent when the exception reaches the caller.
 """
 from collections import OrderedDict
 from typing import Callable, Dict, List, Optional, Tuple
@@ -173,6 +177,11 @@ class RolloutGraph:
     signature, and after every window, eager or replayed, run() extends its rewbuffer / lenbuffer by the episodes the
     window finished, with no sync beyond its one.
 
+    finite_guard (a FiniteGuard whose record(k) `body` calls): its table, workspace and field addresses join the graph
+    signature.  run() zeroes the table before every window and, after the window's bookkeeping (counter, storage.step,
+    episode statistics, extras), raises NonFiniteError when a step flagged a field; step k's events carry
+    common_step_counter = c + k + 1 for a window that started at c.
+
     capture_schedule=True: push and command-curriculum steps are captured too (graphs are cached by the positions of
     the window's disturbance, push and curriculum steps), so after the warm-up every window replays.  For every window
     run() executes, eager or replayed, the env is in its device-schedule mode: the kernels read the command ranges
@@ -183,7 +192,7 @@ class RolloutGraph:
 
     def __init__(self, env, body: Callable[[int], None], num_steps: int, storage=None,
                  finish: Optional[Callable[[], None]] = None, max_graphs: int = 8, warmup: int = 1,
-                 capture_schedule: bool = False, amp=None, episode_stats=None):
+                 capture_schedule: bool = False, amp=None, episode_stats=None, finite_guard=None):
         if not env._kernel_reset_ok():
             raise ValueError("capture_rollout needs the in-kernel reset (a torch reset hook syncs on the host every step)")
         if getattr(env, "gym", None) is not None:
@@ -192,11 +201,15 @@ class RolloutGraph:
             raise ValueError("num_steps must be positive")
         if episode_stats is not None and episode_stats.num_envs != env.num_envs:
             raise ValueError(f"episode_stats keeps {episode_stats.num_envs} envs, the env has {env.num_envs}")
+        if finite_guard is not None and (finite_guard.env is not env or finite_guard.num_steps != num_steps):
+            raise ValueError(f"finite_guard covers {finite_guard.num_steps} steps of another env or rollout length; "
+                             f"the rollout has {num_steps}")
         self.env, self.body, self.num_steps, self.storage, self.finish = env, body, int(num_steps), storage, finish
         self.max_graphs, self.warmup = max(int(max_graphs), 1), int(warmup)
         self.capture_schedule = bool(capture_schedule)
         self.amp = amp
         self.episode_stats = episode_stats
+        self.finite_guard = finite_guard
         self.tables = EpisodeTables(env, self.num_steps)
         self._graphs = OrderedDict()           # key -> (graph, signature, host state after the rollout)
         self._device_counter = None            # what env._step_base holds, when known
@@ -212,7 +225,8 @@ class RolloutGraph:
         return (bytes(env._reset_struct()), noise, env.obs_buf.data_ptr(), env.privileged_obs_buf.data_ptr(),
                 st.step if st is not None else None, env.resample_interval,
                 self.amp.signature() if self.amp is not None else None,
-                self.episode_stats.signature() if self.episode_stats is not None else None)
+                self.episode_stats.signature() if self.episode_stats is not None else None,
+                self.finite_guard.signature() if self.finite_guard is not None else None)
 
     def _host_state(self):
         env, st = self.env, self.storage
@@ -284,6 +298,9 @@ class RolloutGraph:
         env._device_schedule = device_schedule
         if self.amp is not None:
             self.amp.refresh()
+        guard = self.finite_guard
+        if guard is not None:
+            guard.table.zero_()
         try:
             if key is None:
                 self._steps()
@@ -321,10 +338,17 @@ class RolloutGraph:
             env._device_schedule = False
         if self.episode_stats is not None:
             self.episode_stats._enqueue_copies()     # completed by the sync in episode_infos
+        if guard is not None:
+            guard._enqueue_copy()
         infos = self.tables.episode_infos(env, schedule)
         if self.episode_stats is not None:
             self.episode_stats._extend()
         env.extras["time_outs"] = env.time_out_buf
         if infos:
             env.extras["episode"] = infos[-1]
+        if guard is not None:
+            events = guard._events([c + k + 1 for k in range(T)])
+            if events:
+                from .finite_guard import NonFiniteError
+                raise NonFiniteError(events)
         return infos
